@@ -343,6 +343,32 @@ def cuda_eager_reference(cfg, sd, B, L, dev, reps=3):
                 "kernels the reference modules call) on cuda, eager, allow_tf32=False, same batch; context, not the reference arm")
 
 
+DUMP_LIMIT_BYTES = 63_000_000          # 64 MB with room for the .npy headers
+
+
+def sample_outputs(outs, limit=DUMP_LIMIT_BYTES):
+    """outs: {name: device tensor} of one step, clips on axis 1 for "codes" ([n_q, B, T]) and axis 0 otherwise -> {name: float32
+    numpy array}.  Code indices are exact in float32.  When the whole batch exceeds `limit` bytes, the same fixed seeded sample
+    of clips is taken from every array and its indices are returned as "clip_index"."""
+    import torch
+    axis = {name: 1 if name == "codes" else 0 for name in outs}
+    B = outs["codes"].shape[1]
+    per_clip = sum(t.numel() // t.shape[axis[n]] for n, t in outs.items()) * 4
+    clips = None
+    if B * per_clip > limit:
+        keep = max(1, (limit - 8 * B) // per_clip)
+        clips = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    res = {}
+    for name, t in outs.items():
+        t = t.detach().cpu()
+        if clips is not None:
+            t = t.index_select(axis[name], clips)
+        res[name] = t.to(torch.float32).numpy()
+    if clips is not None:
+        res["clip_index"] = clips.to(torch.float32).numpy()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -357,7 +383,14 @@ def main():
     ap.add_argument("--e2e-mode", choices=["sharded-host", "scatter"], default="sharded-host",
                     help="N > 1 end-to-end leg: every rank round-trips its own pinned host shard (default; the reference's "
                          "multi-process inference), or rank 0 holds the whole batch and scatters / gathers it over NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed on rank 0 (codes, quant, scale, recon) as DIR/<name>.npy in "
+                         "float32; when they exceed 64 MB, a fixed seeded sample of clips (listed in DIR/clip_index.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -447,6 +480,8 @@ def main():
     launches = model.launch_count() - launches0
     phases = model.phase_ms()           # the last timed step's phase durations
     model.set_profiling(False)
+    # later legs reuse these buffers: keep the last timed step's outputs now, write them at the end
+    dumped = sample_outputs(dict(codes=codes, quant=quant, scale=scale, recon=recon)) if args.dump_outputs and rank == 0 else None
     clocks = sampler.stop() if rank == 0 else None
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -589,6 +624,11 @@ def main():
                     roofline=roofline, cpu_baseline=cpu, phase_ms_last_step=phases, extra=extra,
                     reference_arm_note=("the --impl reference arm is ONE CPU process (rank 0) at every N: a ratio of this N-GPU "
                                         "aggregate to it scales with N by construction" if world > 1 else None))
+        if dumped is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if world > 1:

@@ -102,24 +102,61 @@ def test_config_from_reference_like_freqcodec():
         config_from_reference_model(m)
 
 
-REF = "/root/reference"
+def reference_description():
+    """tests/golden/reference_modules.json.gz: the reference's own module trees, attributes and state_dict shapes
+    (tools/gen_golden_reference_modules.py)."""
+    import gzip
+    import json
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "reference_modules.json.gz"), "rt") as f:
+        return json.load(f)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout only exists in the build container")
-def test_config_from_the_real_reference_modules():
-    """integration.config_from_reference_model + state_dict name coverage on the REAL reference `Encodec` (ds640, ds320; built by
-    tools/ref_harness.py from /root/reference): every field matches the preset, every tensor the engine needs is in the
-    reference's state_dict under the same name and shape, and option variants that keep the shapes are refused."""
-    import sys
+def rebuild_reference_encodec(desc):
+    """A stand-in for the reference `Encodec` rebuilt from its recorded description: encoder / decoder module trees with the
+    recorded class names and attributes (torch's own GroupNorm / ELU / Sequential where the reference uses them), the
+    quantizer attributes, and a state_dict of meta tensors with the recorded names and shapes."""
+    import types
     import torch
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    from ref_harness import build_reference_encodec
+    import torch.nn as nn
+    classes = {}
+
+    def make(cls, attrs):
+        if cls == "GroupNorm":
+            return nn.GroupNorm(attrs["num_groups"], attrs["num_channels"], attrs["eps"], attrs["affine"])
+        if cls == "ELU":
+            return nn.ELU(attrs["alpha"])
+        mod = nn.Sequential() if cls == "Sequential" else classes.setdefault(cls, type(cls, (nn.Module,), {}))()
+        for k, v in attrs.items():
+            setattr(mod, k, v)
+        return mod
+
+    def tree(entries):
+        root = make(entries[0][1], entries[0][2])
+        for path, cls, attrs in entries[1:]:
+            parent, _, leaf = path.rpartition(".")
+            root.get_submodule(parent).add_module(leaf, make(cls, attrs))
+        return root
+
+    sd = {k: torch.empty(shape, device="meta") for k, shape in desc["state_dict"].items()}
+    return types.SimpleNamespace(
+        encoder=tree(desc["encoder"]), decoder=tree(desc["decoder"]),
+        quantizer=types.SimpleNamespace(rq=types.SimpleNamespace(model=types.SimpleNamespace(**desc["rq_model"])),
+                                        **desc["quantizer"]),
+        state_dict=lambda: sd, **desc["attrs"])
+
+
+def test_config_from_the_real_reference_modules():
+    """integration.config_from_reference_model + state_dict name coverage on the REAL reference `Encodec` (as recorded in
+    tests/golden/reference_modules.json.gz from the models tools/ref_harness.py builds): every field matches the preset, every
+    tensor the engine needs is in the reference's state_dict under the same name and shape, and option variants that keep
+    the shapes are refused."""
     from funcodec_b200.integration import config_from_reference_model, stacked_codebooks, UnsupportedReferenceModel
     from funcodec_b200.weights import state_dict_shapes
+    models = reference_description()["models"]
     for name in ("encodec_16k_n32_ds320", "tiny_ds40", "soundstream_noncausal_small", "soundstream_causal_small",
                  "weightnorm_lstm_small"):
         cfg = get_config(name)
-        m = build_reference_encodec(cfg)
+        m = rebuild_reference_encodec(models[name])
         got = config_from_reference_model(m)
         for f in ("arch", "ratios", "n_filters", "dimension", "kernel_size", "last_kernel_size", "residual_kernel_size",
                   "lstm_layers", "codebook_size", "num_quantizers", "sample_rate", "audio_normalize", "n_residual_layers",
@@ -130,7 +167,7 @@ def test_config_from_the_real_reference_modules():
             assert k in sd and tuple(sd[k].shape) == tuple(shp), (name, k)
         assert tuple(stacked_codebooks(sd).shape) == (cfg.num_quantizers, cfg.codebook_size, cfg.dimension)
     # options that keep parameter names and shapes but change the maths are refused
-    m = build_reference_encodec(get_config("tiny_ds40"))
+    m = rebuild_reference_encodec(models["tiny_ds40"])
     m.encoder.model[0].causal = True                   # one causal conv among non-causal ones / causal under GroupNorm
     with pytest.raises(UnsupportedReferenceModel):
         config_from_reference_model(m)
@@ -144,22 +181,16 @@ def test_config_from_the_real_reference_modules():
         config_from_reference_model(m)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout only exists in the build container")
 def test_use_ddp_false_reference_quantizer_keys():
     """`use_ddp: false` (core_vq.py:147-150): the reference's own per-layer key names are what stacked_codebooks / fcb_finalize
     assemble into the [n_q, K, D] codebook tensor."""
-    import sys
     import torch
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    from ref_harness import import_reference
-    import_reference()
-    from funcodec.modules.quantization.core_vq import ResidualVectorQuantization
     from funcodec_b200.integration import stacked_codebooks
-    # (in this checkout CostumeQuantizer(use_ddp=False) itself raises -- vq.py:73-84 passes q0_ds_ratio, which
-    # core_vq.VectorQuantization does not accept -- so the RVQ class is built directly; it sits at quantizer.rq.model)
-    rvq = ResidualVectorQuantization(num_quantizers=3, dim=16, codebook_size=32, decay=0.99, kmeans_init=True, kmeans_iters=10,
-                                     threshold_ema_dead_code=2, quantize_dropout=True, rand_num_quant=[1, 2, 3])
-    sd = {"quantizer.rq.model." + k: v for k, v in rvq.state_dict().items()}
+    # (in the reference CostumeQuantizer(use_ddp=False) itself raises -- vq.py:73-84 passes q0_ds_ratio, which
+    # core_vq.VectorQuantization does not accept -- so the fixture records the RVQ class built directly
+    # (3 layers, dim 16, 32 codes); it sits at quantizer.rq.model)
+    keys = reference_description()["rvq_use_ddp_false"]
+    sd = {"quantizer.rq.model." + k: torch.zeros(shape) for k, shape in keys.items()}
     assert "quantizer.rq.model.layers.0._codebook.embed" in sd and "quantizer.rq.model.embed" not in sd
     for i in range(3):
         sd[f"quantizer.rq.model.layers.{i}._codebook.embed"] = torch.full((32, 16), float(i))

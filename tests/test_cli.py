@@ -15,7 +15,6 @@ from funcodec_b200.bin import codec_inference as CLI
 from funcodec_b200.kaldi_io import ArkScpWriter, read_mat, read_scp_mats
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_CONF = "/root/reference/egs/LibriTTS/codec/conf"
 
 
 def stage_argv(stage, d, job=1, batch_size=4, bit_width=16000, indices_save_type="text", sr=16000):
@@ -106,19 +105,26 @@ def test_config_from_yaml_refuses_unbuilt_conv_options(tmp_path, patch):
         CLI.config_from_yaml(path)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONF), reason="the reference checkout only exists in the build container")
-def test_config_from_the_reference_repo_yamls():
-    """The YAMLs the reference ships: the two Encodec ones, the two mag_phase FreqCodec ones, the two non-causal SoundStream ones
-    (3 dilated residual blocks per stage, no sequence model) and the causal weight_norm SoundStream one map to presets; the
-    mag_angle FreqCodec one is refused with a message."""
+def test_config_from_the_reference_repo_yamls(tmp_path):
+    """The YAMLs the reference ships (egs/LibriTTS/codec/conf, as recorded in tests/golden/reference_modules.json.gz): the two
+    Encodec ones, the two mag_phase FreqCodec ones, the two non-causal SoundStream ones (3 dilated residual blocks per stage,
+    no sequence model) and the causal weight_norm SoundStream one map to presets; the mag_angle FreqCodec one is refused with
+    a message."""
+    import gzip
+    import yaml
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "reference_modules.json.gz"), "rt") as f:
+        confs = json.load(f)["yaml_conf"]
+    assert len(confs) == 8
     want = {"encodec_16k_n32_600k_step.yaml": "encodec_16k_n32_ds320", "encodec_16k_n32_600k_step_ds640.yaml": "encodec_16k_n32_ds640",
             "soundstream_noncausal_16k_n32_600k_step.yaml": "soundstream_noncausal_16k_n32_ds320",
             "soundstream_noncausal_16k_n32_600k_step_ds640.yaml": "soundstream_noncausal_16k_n32_ds640",
             "soundstream_16k_n32_600k_step.yaml": "soundstream_16k_n32_ds320",
             "freqcodec_mag_phase_16k_n32_600k_step.yaml": "freqcodec_magphase_16k_n32_ds320",
             "freqcodec_mag_phase_16k_n32_600k_step_ds640.yaml": "freqcodec_magphase_16k_n32_ds640"}
-    for fn in sorted(os.listdir(REF_CONF)):
-        path = os.path.join(REF_CONF, fn)
+    for fn in sorted(confs):
+        path = os.path.join(tmp_path, fn)
+        with open(path, "wt") as f:
+            yaml.safe_dump(confs[fn], f)
         if fn in want:
             got, _, _ = CLI.config_from_yaml(path)
             cfg = get_config(want[fn])
