@@ -57,19 +57,8 @@ struct ConvParams {
     int T_out, C_out;
     long long out_clip_stride;
     double* partials;        // [B][n_parts][2] (sum, sum of squares) or nullptr
-    // fused GroupNorm finalisation (conv_tc.cu): the CTA that writes a clip's LAST partial reduces them (fixed order) into
-    // (mean, rstd) + the per-channel affine, so no separate stats_finalize launch is needed.  fin_counter == nullptr: disabled.
-    int* fin_counter;        // [clips] zero between launches (the finalising CTA resets its clip's entry)
-    float* fin_stats;        // [clips][2]
-    float* fin_coef;         // [clips][2][fin_C]
-    const float* fin_gamma;
-    const float* fin_beta;
-    int fin_C, fin_parts;    // channels of the affine; partials per clip (2-D: F_out x per-row partials)
-    double fin_count;        // elements per clip
-    float fin_eps;
     int cic;                 // input-channel chunk staged per iteration
     Freq2d fq;               // tensor-core 2-D mode (zero-initialised for 1-D layers)
-    int dbg;                 // PROFILING ONLY (env FCB_TC_DBG, conv_tc.cu): knock-out mask; results are wrong when != 0
 };
 
 // ---- FreqCodec 2-D path (conv2d_simt.cu): raw activations are channels-last [B][F_raw][T_raw][C]

@@ -41,7 +41,6 @@
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_sm100.cuh"
-#include <stdlib.h>
 
 namespace fcb {
 
@@ -233,18 +232,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                 uint8_t* hi = smA + as * L.a_stage;
                 uint8_t* lo = hi + L.a_rows * 128;
                 const uint32_t c16 = (uint32_t)(half * 4 + (jchunk >> 1)), sub8 = (uint32_t)((jchunk & 1) << 3);
-                if (p.dbg & 512) {
-                    if (p.dbg & 64) mbar_wait(a_empty + as, par); else mbar_wait_backoff(a_empty + as, par, 64);
-                } else if (chunk >= n_chunks) {
-                    if (p.dbg & 64) mbar_wait(a_empty + as, par); else mbar_wait_backoff(a_empty + as, par, 64);      // missing half of the last stage: never read by the MMAs
+                if (chunk >= n_chunks) {
+                    mbar_wait_backoff(a_empty + as, par, 64);      // missing half of the last stage: never read by the MMAs
                 } else if (interior) {
                     // ---- TMA-staged unit: the dense [a_rows][32 ch] boxes (+ the coefficient slices) wait in the raw ring; rows go
                     // shared -> registers -> shared one at a time (no long-latency loads to batch, few live registers)
-                    bool c_ok = chunk * TC_KC + jchunk * 4 < C_in;
-                    if (FREQ && p.pad_zero) {              // a zero-padded frequency tap contributes nothing (its box arrives zero-filled)
-                        const int f_src = f_out * p.fq.SF + (chunk * TC_KC) / pitch - p.fq.pad_f;
-                        c_ok = c_ok && f_src >= 0 && f_src < p.fq.F_in;
-                    }
+                    const bool c_ok = chunk * TC_KC + jchunk * 4 < C_in;
                     const int idx = 2 * S * sc + ((2 * sc + 1 < n_chunks) ? 2 * ph + half : ph);
                     const int rc = rawbase + idx;
                     const int rslot = rc % nraw;
@@ -264,7 +257,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                             b1.x *= in_scale; b1.y *= in_scale; b1.z *= in_scale; b1.w *= in_scale;
                         }
                     }
-                    if (p.dbg & 64) mbar_wait(a_empty + as, par); else mbar_wait_backoff(a_empty + as, par, 64);
+                    mbar_wait_backoff(a_empty + as, par, 64);
                     const uint8_t* rrow = rb + rsub * raw_pitch + jchunk * 16;
 #pragma unroll
                     for (int i = 0; i < 5; ++i) {
@@ -285,7 +278,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                                     v.z = elu_scaled(v.z, p.tc_elu_k, in_scale); v.w = elu_scaled(v.w, p.tc_elu_k, in_scale);
                                 }
                             }
-                            if (p.dbg & 4) continue;
                             uint2 h, l;
                             split_f16x2(v.x, v.y, h.x, l.x);
                             split_f16x2(v.z, v.w, h.y, l.y);
@@ -340,20 +332,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                     okr[i] = ok;
                     xa[i] = make_float4(0.f, 0.f, 0.f, 0.f);
                     xb[i] = xa[i];
-                    if (ok && !(p.dbg & 1)) {
+                    if (ok) {
                         const long long off = (long long)src * pitch + c;
                         xa[i] = __ldg(reinterpret_cast<const float4*>(xu0 + off));
                         if (has1) xb[i] = __ldg(reinterpret_cast<const float4*>(xu1 + off));
                     }
                 }
-                if (p.dbg & 64) mbar_wait(a_empty + as, par); else mbar_wait_backoff(a_empty + as, par, 64);
+                mbar_wait_backoff(a_empty + as, par, 64);
 #pragma unroll
                 for (int i = 0; i < NR; ++i) {
                     const int u = rsub + 32 * i;
                     if (u < L.a_rows) {
                         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (p.dbg & 2) v = xa[i];
-                        else if (okr[i]) {
+                        if (okr[i]) {
                             const float4 xv = xa[i];
                             v.x = fmaf(xv.x, a0.x, b0.x); v.y = fmaf(xv.y, a0.y, b0.y);
                             v.z = fmaf(xv.z, a0.z, b0.z); v.w = fmaf(xv.w, a0.w, b0.w);
@@ -367,7 +358,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                                 v.z = elu_scaled(v.z, p.tc_elu_k, in_scale); v.w = elu_scaled(v.w, p.tc_elu_k, in_scale);
                             }
                         }
-                        if (p.dbg & 4) continue;
                         uint2 h, l;
                         split_f16x2(v.x, v.y, h.x, l.x);
                         split_f16x2(v.z, v.w, h.y, l.y);
@@ -402,12 +392,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                 int chunk = 0, ph = 0;                                 // chunk: 64-channel stage chunk
                 for (int unit = 0; unit < n_units; ++unit) {
                     for (int k = ph; k < K; k += S) {
-                        if (!w_resident) { if (p.dbg & 64) mbar_wait(b_empty + bs, bphase ^ 1); else mbar_wait_backoff(b_empty + bs, bphase ^ 1, 64); }
-                        if (p.dbg & 256) { mbar_arrive(b_full + bs); }
-                        else {
-                            mbar_arrive_expect_tx(b_full + bs, bytes);
-                            bulk_g2s(smB + bs * L.b_stage, wbase + ((long long)chunk * K + k) * bytes, bytes, b_full + bs);
-                        }
+                        if (!w_resident) mbar_wait_backoff(b_empty + bs, bphase ^ 1, 64);
+                        mbar_arrive_expect_tx(b_full + bs, bytes);
+                        bulk_g2s(smB + bs * L.b_stage, wbase + ((long long)chunk * K + k) * bytes, bytes, b_full + bs);
                         if (++bs == nb_stages) { bs = 0; bphase ^= 1; }
                     }
                     if (++ph == S) { ph = 0; ++chunk; }
@@ -447,7 +434,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                             }
                             const uint32_t b_hi0 = b_base + bs * L.b_stage;
                             const uint32_t b_lo0 = b_hi0 + N_TILE * 128;
-                            if (!(p.dbg & 32))
 #pragma unroll
                             for (int ks = 0; ks < 4; ++ks) {
                                 if (ks < ksteps) {
@@ -476,7 +462,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
         }
     } else if (warp == 22) {
         // =========================================================== raw activation tiles via TMA (cp.async.bulk.tensor)
-        if (lane == 0 && nraw > 0 && !(p.dbg & 512)) {
+        if (lane == 0 && nraw > 0) {
             const uint32_t row_bytes = (uint32_t)(L.a_rows * raw_pitch);
             const uint32_t cbytes = (uint32_t)raw_pitch;
             const uint32_t n_cf = (p.in0.coef ? 2u : 0u) + ((has1 && p.in1.coef) ? 2u : 0u);
@@ -486,11 +472,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                 const TcTile tl = tc_tile(tile, n_nt, n_tt);
                 const int t0 = tl.tt * TC_M;
                 if (!tile_interior(t0)) continue;
-                int b = tl.b, f_out = 0;
-                if (FREQ) { b = tl.b / p.fq.F_out; f_out = tl.b - b * p.fq.F_out; }
-                const int pitch = FREQ ? p.fq.cin : C_in;
-                const float* cf0 = p.in0.coef ? p.in0.coef + (long long)b * 2 * pitch : nullptr;
-                const float* cf1 = (has1 && p.in1.coef) ? p.in1.coef + (long long)b * 2 * pitch : nullptr;
+                const int b = tl.b;
+                const float* cf0 = p.in0.coef ? p.in0.coef + (long long)b * 2 * C_in : nullptr;
+                const float* cf1 = (has1 && p.in1.coef) ? p.in1.coef + (long long)b * 2 * C_in : nullptr;
                 for (int sc = 0; sc < n_sc; ++sc)
                     for (int ph = 0; ph < S; ++ph) {
                         // row (t0 + u) * S + ph - pad_l == (tq0 + u) * S + php
@@ -504,27 +488,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                             mbar_wait(raw_empty + slot, (uint32_t)((rc / nraw) & 1) ^ 1);
                             uint8_t* dst = smR + slot * L.raw_slot;
                             mbar_arrive_expect_tx(raw_full + slot, unit_bytes);
-                            int c0 = chunk * TC_KC;            // first stored channel of the unit
-                            if (FREQ) {
-                                // gathered chunk -> (frequency tap, 32-channel slice of it); a reflected tap is just another row,
-                                // a zero-padded one is out of bounds for the tensor map (zero fill)
-                                const int kf = c0 / pitch;
-                                c0 -= kf * pitch;
-                                int f_src = f_out * p.fq.SF + kf - p.fq.pad_f;
-                                if (!p.pad_zero) f_src = reflect_index(f_src, p.fq.F_in);
-                                tma_load_5d(dst, &tm0, c0, php, tq0, f_src, b, raw_full + slot);
-                                if (has1) tma_load_5d(dst + L.raw_in1, &tm1, c0, php, tq0, f_src, b, raw_full + slot);
-                            } else {
-                                tma_load_4d(dst, &tm0, c0, php, tq0, b, raw_full + slot);
-                                if (has1) tma_load_4d(dst + L.raw_in1, &tm1, c0, php, tq0, b, raw_full + slot);
-                            }
+                            const int c0 = chunk * TC_KC;      // first channel of the unit
+                            tma_load_4d(dst, &tm0, c0, php, tq0, b, raw_full + slot);
+                            if (has1) tma_load_4d(dst + L.raw_in1, &tm1, c0, php, tq0, b, raw_full + slot);
                             if (cf0) {
                                 bulk_g2s(dst + L.raw_cf, cf0 + c0, cbytes, raw_full + slot);
-                                bulk_g2s(dst + L.raw_cf + 128, cf0 + pitch + c0, cbytes, raw_full + slot);
+                                bulk_g2s(dst + L.raw_cf + 128, cf0 + C_in + c0, cbytes, raw_full + slot);
                             }
                             if (cf1) {
                                 bulk_g2s(dst + L.raw_cf + 256, cf1 + c0, cbytes, raw_full + slot);
-                                bulk_g2s(dst + L.raw_cf + 384, cf1 + pitch + c0, cbytes, raw_full + slot);
+                                bulk_g2s(dst + L.raw_cf + 384, cf1 + C_in + c0, cbytes, raw_full + slot);
                             }
                             ++rc;
                         }
@@ -541,54 +514,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
         // 2-D plain convs (no phase scatter, no padded columns) store [pseudo-clip][t][C_out] like a 1-D layer
         const bool plain_out = FREQ && p.fq.FR == 1 && p.fq.TR == 1 && p.fq.c_store == p.C_out;
         const float out_scale = p.tc_out_scale;
-        // fused GroupNorm finalisation: partials of the current clip written by this CTA since the last report
-        int fin_clip = -1, fin_local = 0;
-        auto fin_flush = [&]() {
-            // all 128 accumulator threads call this together.  Report this CTA's partial count for fin_clip; whoever completes the
-            // clip reduces ALL its partials in a fixed order (independent of which CTA does it) and writes stats + affine.
-            if (fin_clip < 0 || fin_local == 0) return;
-            int* flag = reinterpret_cast<int*>(red + 8);
-            if (quad == 0 && lane == 0) {
-                __threadfence();                                         // this CTA's partials before the count
-                const int old = atomicAdd(p.fin_counter + fin_clip, fin_local);
-                *flag = (old + fin_local == p.fin_parts) ? 1 : 0;
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-            const bool last_cta = *flag != 0;
-            if (last_cta) {
-                __threadfence();                                         // the other CTAs' partials after the count
-                const int t128 = quad * 32 + lane;
-                const double* pp = p.partials + (long long)fin_clip * p.fin_parts * 2;
-                double fs = 0.0, fss = 0.0;
-                for (int i = t128; i < p.fin_parts; i += 128) { fs += __ldcg(pp + 2 * i); fss += __ldcg(pp + 2 * i + 1); }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    fs += __shfl_xor_sync(0xffffffffu, fs, o);
-                    fss += __shfl_xor_sync(0xffffffffu, fss, o);
-                }
-                asm volatile("bar.sync 1, 128;" ::: "memory");          // everyone has read the flag
-                if (lane == 0) { red[quad * 2] = fs; red[quad * 2 + 1] = fss; }
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                const double ts = (red[0] + red[2]) + (red[4] + red[6]), tss = (red[1] + red[3]) + (red[5] + red[7]);
-                const double mean_d = ts / p.fin_count;
-                double var = tss / p.fin_count - mean_d * mean_d;
-                if (var < 0.0) var = 0.0;
-                const float mean = (float)mean_d, rstd = (float)(1.0 / sqrt(var + (double)p.fin_eps));
-                if (t128 == 0) {
-                    p.fin_stats[2 * fin_clip] = mean;
-                    p.fin_stats[2 * fin_clip + 1] = rstd;
-                    p.fin_counter[fin_clip] = 0;                         // ready for the next launch
-                }
-                if (p.fin_coef)
-                    for (int c = t128; c < p.fin_C; c += 128) {
-                        const float a = rstd * p.fin_gamma[c];
-                        p.fin_coef[(long long)fin_clip * 2 * p.fin_C + c] = a;
-                        p.fin_coef[(long long)fin_clip * 2 * p.fin_C + p.fin_C + c] = p.fin_beta[c] - a * mean;
-                    }
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");              // `red` / flag free again
-            fin_local = 0;
-        };
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             const TcTile tl = tc_tile(tile, n_nt, n_tt);
             const int t = tl.tt * TC_M + quad * 32 + lane;
@@ -603,9 +528,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
             float s = 0.f, ss = 0.f;
             for (int g = 0; g < n_groups; ++g) {
                 const bool last = (g == n_groups - 1);
-                if (p.dbg & 64) mbar_wait(acc_full + buf, cphase); else mbar_wait_backoff(acc_full + buf, cphase, 128);
+                mbar_wait_backoff(acc_full + buf, cphase, 128);
                 tc_fence_after_sync();
-                if (!(p.dbg & 128))
 #pragma unroll
                 for (int c0 = 0; c0 < N_TILE; c0 += 32) {
                     uint32_t v[32];
@@ -641,18 +565,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                             }
                         }
                         __syncwarp();
-                        if (!(p.dbg & 8)) {
-                            const int cc = lane & 7;
-                            if (c0 + cc * 4 < N_TILE) {
-                                float* obase = p.out + (long long)tl.b * p.out_clip_stride + (long long)tl.nt * N_TILE + c0 + cc * 4;
-                                const int trow0 = tl.tt * TC_M + quad * 32;
+                        const int cc = lane & 7;
+                        if (c0 + cc * 4 < N_TILE) {
+                            float* obase = p.out + (long long)tl.b * p.out_clip_stride + (long long)tl.nt * N_TILE + c0 + cc * 4;
+                            const int trow0 = tl.tt * TC_M + quad * 32;
 #pragma unroll
-                                for (int i = 0; i < 8; ++i) {
-                                    const int rr = i * 4 + (lane >> 3);
-                                    if (trow0 + rr < p.T_out)
-                                        *reinterpret_cast<float4*>(obase + (long long)(trow0 + rr) * p.C_out) =
-                                            *reinterpret_cast<const float4*>(stg + rr * 128 + ((cc ^ (rr & 7)) << 4));
-                                }
+                            for (int i = 0; i < 8; ++i) {
+                                const int rr = i * 4 + (lane >> 3);
+                                if (trow0 + rr < p.T_out)
+                                    *reinterpret_cast<float4*>(obase + (long long)(trow0 + rr) * p.C_out) =
+                                        *reinterpret_cast<const float4*>(stg + rr * 128 + ((cc ^ (rr & 7)) << 4));
                             }
                         }
                         __syncwarp();
@@ -674,22 +596,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                                 o.w = fmaf(__uint_as_float(v[j + 3]), out_scale, __ldg(bias + c0 + j + 3));
                                 s += (o.x + o.y) + (o.z + o.w);
                                 ss = fmaf(o.x, o.x, ss); ss = fmaf(o.y, o.y, ss); ss = fmaf(o.z, o.z, ss); ss = fmaf(o.w, o.w, ss);
-                                if (p.dbg & 8) {
-                                } else {
-                                    // phase (pf, pt) of a transposed conv lands on row f_out*FR + pf, column t*TR + pt
-                                    const int pf = ph / p.fq.TR, pt = ph - pf * p.fq.TR;
-                                    float* dst = p.out + (frow + (long long)pf * p.T_out * p.fq.TR + pt) * p.fq.c_store + cch;
-                                    if ((p.fq.c_store & 3) == 0) {
-                                        if (cch < p.fq.c_store) *reinterpret_cast<float4*>(dst) = o;   // (padded columns: no store)
-                                    } else {                          // padded n-tile: only the real channels exist in HBM
-                                        if (cch + 0 < p.fq.c_store) dst[0] = o.x;
-                                        if (cch + 1 < p.fq.c_store) dst[1] = o.y;
-                                        if (cch + 2 < p.fq.c_store) dst[2] = o.z;
-                                        if (cch + 3 < p.fq.c_store) dst[3] = o.w;
-                                    }
-                                    cch += 4;
-                                    if (cch >= p.fq.Cc) { cch = 0; ++ph; }
+                                // phase (pf, pt) of a transposed conv lands on row f_out*FR + pf, column t*TR + pt
+                                const int pf = ph / p.fq.TR, pt = ph - pf * p.fq.TR;
+                                float* dst = p.out + (frow + (long long)pf * p.T_out * p.fq.TR + pt) * p.fq.c_store + cch;
+                                if ((p.fq.c_store & 3) == 0) {
+                                    if (cch < p.fq.c_store) *reinterpret_cast<float4*>(dst) = o;   // (padded columns: no store)
+                                } else {                          // padded n-tile: only the real channels exist in HBM
+                                    if (cch + 0 < p.fq.c_store) dst[0] = o.x;
+                                    if (cch + 1 < p.fq.c_store) dst[1] = o.y;
+                                    if (cch + 2 < p.fq.c_store) dst[2] = o.z;
+                                    if (cch + 3 < p.fq.c_store) dst[3] = o.w;
                                 }
+                                cch += 4;
+                                if (cch >= p.fq.Cc) { cch = 0; ++ph; }
                             }
                         }
                     }
@@ -699,7 +618,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                 mbar_arrive(acc_empty + buf);
                 if (++buf == n_acc) { buf = 0; cphase ^= 1; }
             }
-            if (p.partials && !(p.dbg & 16)) {
+            if (p.partials) {
                 double ds = (double)s, dss = (double)ss;
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) {
@@ -715,14 +634,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv1d_tc_kernel(const __grid_c
                     dst[0] = (red[0] + red[2]) + (red[4] + red[6]);
                     dst[1] = (red[1] + red[3]) + (red[5] + red[7]);
                 }
-                if (p.fin_counter) {
-                    const int clip = FREQ ? tl.b / p.fq.F_out : tl.b;
-                    if (clip != fin_clip) { fin_flush(); fin_clip = clip; }
-                    ++fin_local;
-                }
             }
         }
-        if (p.fin_counter && p.partials && !(p.dbg & 16)) fin_flush();
     }
     tc_fence_before_sync();
     __syncthreads();
@@ -772,19 +685,16 @@ int conv_tc_num_parts(int T_out, int C_out_eff) {
 
 static int g_num_sms = 0;
 
-static int g_group_mmas = TC_GROUP_MMAS, g_deep_ring = 1, g_dbg = 0, g_nacc_cap = 0, g_na_tma = 2;
-
 struct TcPlan { int resident, na, nb, nraw; TcSmemLayout L; bool ok; };
 
 // shared-memory plan: weights resident (small layers: the whole image of the single n-tile) or streamed through a ring as
 // deep as fits; A ring `na_first` stages (4, else 2) -- with a raw TMA ring the A ring only decouples producers from the MMA
 // issue, so 2 stages suffice and the rest of the shared memory buys prefetch depth (nraw units in flight).
-static TcPlan tc_plan(const ConvParams& p, int na_first, bool want_raw, int g_deep_ring) {
+static TcPlan tc_plan(const ConvParams& p, int na_first, bool want_raw) {
     const int limit = 225 * 1024;
     const int n_slabs = ((p.C_in + 2 * TC_KC - 1) / (2 * TC_KC)) * p.K;   // (64-channel stage chunk, tap) weight slabs per n-tile
     const int has1 = p.in1.x ? 1 : 0;
-    const int cin_row = p.fq.KF > 0 ? p.fq.cin : p.C_in;                   // channels of a stored input row
-    const int raw_pitch = (cin_row < TC_KC ? cin_row : TC_KC) * 4;
+    const int raw_pitch = (p.C_in < TC_KC ? p.C_in : TC_KC) * 4;           // raw ring: 1-D layers only
     TcPlan pl{};
     pl.ok = false;
     int na = na_first, nb = 4;
@@ -800,7 +710,7 @@ static TcPlan tc_plan(const ConvParams& p, int na_first, bool want_raw, int g_de
         if (!fits(L)) { nb = 2; L = tc_layout(p.K, p.S, p.n_tile, na, nb); }
         if (!fits(L)) return pl;
         // small n-tiles: a weight slab is only n_tile*256 bytes, so the ring is deepened until shared memory is full
-        if (g_deep_ring && !want_raw)
+        if (!want_raw)
             while (nb < 24 && nb < n_slabs && tc_layout(p.K, p.S, p.n_tile, na, nb + 1).total <= limit)
                 L = tc_layout(p.K, p.S, p.n_tile, na, ++nb);
     }
@@ -819,7 +729,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn g_encode_tiled = nullptr;
-static int g_tma_state = 0;      // 0: not probed, 1: available, -1: unavailable / disabled (FCB_TC_TMA=0)
+static int g_tma_state = 0;      // 0: not probed, 1: available, -1: unavailable
 
 // 4-D view of a channels-last activation [B][T][C] that makes every stride phase a dimension: (channel, phase, row / S, clip).
 // A unit of a tile = box {32 channels, 1 phase, a_rows rows, 1 clip}; rows beyond T / S (and before 0) are zero-filled.
@@ -831,22 +741,6 @@ static bool make_act_map(CUtensorMap* tm, const InView& v, int C, int S, int T_i
     const cuuint32_t estr[4] = {1, 1, 1, 1};
     if (((uintptr_t)base & 15) != 0 || (strides[0] & 15) || (strides[2] & 15) || dims[2] == 0) return false;
     return g_encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// 2-D (FreqCodec) activation [B][F_raw][T_raw][cin]: (channel, phase, column / ST, frequency row, clip); the logical window
-// starts at (f_off, t_off) and spans F_in x T_in -- taps outside it are out of bounds (zero fill) or reflected by the caller.
-static bool make_act_map_2d(CUtensorMap* tm, const InView& v, int cin, int ST, int T_in, int F_in, int T_raw, int f_off, int B,
-                            int a_rows) {
-    const float* base = v.x + ((long long)f_off * T_raw + v.row_off) * cin;
-    const cuuint64_t dims[5] = {(cuuint64_t)cin, (cuuint64_t)ST, (cuuint64_t)(T_in / ST), (cuuint64_t)F_in, (cuuint64_t)B};
-    const cuuint64_t strides[4] = {(cuuint64_t)cin * 4, (cuuint64_t)ST * cin * 4, (cuuint64_t)T_raw * cin * 4,
-                                   (cuuint64_t)v.clip_stride * 4};
-    const cuuint32_t box[5] = {(cuuint32_t)(cin < TC_KC ? cin : TC_KC), 1, (cuuint32_t)a_rows, 1, 1};
-    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    if (((uintptr_t)base & 15) != 0 || (strides[0] & 15) || (strides[2] & 15) || (strides[3] & 15) || dims[2] == 0) return false;
-    return g_encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<float*>(base), dims, strides, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -866,19 +760,18 @@ static cudaError_t launch_tc_n(const ConvParams& p, cudaStream_t st, const TcPla
     ka.n_sc = (ka.n_chunks + 1) >> 1;
     ka.split = ka.n_chunks > 1;
     ka.n_units = ka.n_sc * p.S;
-    ka.upg = tc_units_per_group(p.K, p.S, g_group_mmas);
+    ka.upg = tc_units_per_group(p.K, p.S, TC_GROUP_MMAS);
     ka.n_groups = (ka.n_units + ka.upg - 1) / ka.upg;
     ka.n_tt = (p.T_out + TC_M - 1) / TC_M;
     ka.n_nt = p.C_out / N_TILE;
     ka.units_per_tile = ka.n_chunks * p.S;
     ka.tq_rows = p.T_in / p.S;
-    ka.raw_pitch = ((FREQ ? p.fq.cin : p.C_in) < TC_KC ? (FREQ ? p.fq.cin : p.C_in) : TC_KC) * 4;
+    ka.raw_pitch = (p.C_in < TC_KC ? p.C_in : TC_KC) * 4;
     // accumulator ring depth: layers whose tile is one accumulation group keep up to 8 tiles in flight between MMA issue and
     // epilogue; layers that fold groups (deep K) ping-pong between up to 3 accumulators next to the running totals
     constexpr int BUF_COLS = N_TILE < 32 ? 32 : N_TILE;
     const int acc_fit = 512 / BUF_COLS;
     ka.n_acc = ka.n_groups == 1 ? (acc_fit < 8 ? acc_fit : 8) : (acc_fit - 1 < 3 ? acc_fit - 1 : 3);
-    if (g_nacc_cap >= 2 && ka.n_acc > g_nacc_cap) ka.n_acc = g_nacc_cap;       // experiments (FCB_TC_NACC)
     kern<<<grid, TC_THREADS, pl.L.total, st>>>(p, ka, tm0, tm1);
     return cudaGetLastError();
 }
@@ -897,26 +790,16 @@ cudaError_t launch_conv_tc(const ConvParams& p_in, int B, cudaStream_t st, int* 
         if (e != cudaSuccess) return e;
         e = cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
         if (e != cudaSuccess) return e;
-        // tuning knobs (experiments only; defaults are the shipped configuration)
-        if (const char* v = getenv("FCB_TC_GROUP_MMAS")) g_group_mmas = atoi(v) > 0 ? atoi(v) : TC_GROUP_MMAS;
-        if (const char* v = getenv("FCB_TC_DEEP_RING")) g_deep_ring = atoi(v) != 0;
-        if (const char* v = getenv("FCB_TC_DBG")) g_dbg = atoi(v);      // profiling knock-outs (wrong results)
-        if (const char* v = getenv("FCB_TC_NACC")) g_nacc_cap = atoi(v);
-        if (const char* v = getenv("FCB_TC_NA_TMA")) { const int f = atoi(v); if (f == 2 || f == 4) g_na_tma = f; }
         // TMA staging of the activation tiles: cuTensorMapEncodeTiled through the runtime's driver entry point (no -lcuda)
         g_tma_state = -1;
-        const char* tv = getenv("FCB_TC_TMA");
-        if (!tv || atoi(tv) != 0) {
-            void* fn = nullptr;
-            cudaDriverEntryPointQueryResult qres;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && fn &&
-                qres == cudaDriverEntryPointSuccess) {
-                g_encode_tiled = (EncodeTiledFn)fn;
-                g_tma_state = 1;
-            }
+        void* fn = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) == cudaSuccess && fn &&
+            qres == cudaDriverEntryPointSuccess) {
+            g_encode_tiled = (EncodeTiledFn)fn;
+            g_tma_state = 1;
         }
     }
-    p.dbg = g_dbg;
     if (!(p.tc_in_scale > 0.f)) p.tc_in_scale = 16.f;           // post-GroupNorm activations are O(1): 16 x keeps |x| < 4094 finite
     if (!(p.tc_w_scale > 0.f)) p.tc_w_scale = 1.f;
     p.tc_out_scale = 1.0f / (p.tc_in_scale * p.tc_w_scale);     // powers of two: exact
@@ -927,29 +810,19 @@ cudaError_t launch_conv_tc(const ConvParams& p_in, int B, cudaStream_t st, int* 
     const bool freq = p.fq.KF > 0;          // B counts pseudo-clips (clips x output frequency rows) in the 2-D mode
     // raw TMA ring: 1-D layers with interior tiles (n_tt >= 3), channel counts the box covers, 16-byte aligned views
     CUtensorMap tm0{}, tm1{};
-    // (2-D: a 32-channel unit must be a slice of ONE frequency tap -> cin % 32 == 0, or the single tap of a 16-channel 1x1 conv)
     // (interior tiles exist when the clip has at least 3 tiles, or for 1x1 layers -- no halo -- always)
-    bool want_raw = g_tma_state == 1 && (n_tt >= 3 || (p.K == 1 && p.S == 1 && p.pad_l == 0)) && p.T_in / p.S >= 1 &&
-                    (freq ? (p.fq.cin % TC_KC == 0 || (p.fq.cin == 16 && p.fq.KF == 1)) : (p.C_in % TC_KC == 0 || p.C_in == 16));
-    // 2-D layers: built and parity-tested (5-D tensor maps), but measured SLOWER than the per-thread gather at config 4 (r2g: conv
-    // stack 37.3 vs 33.6 ms) -- the K_F-fold re-read of every input row makes the unit stream L2-bound either way and the TMA path
-    // adds a hand-off; opt-in (FCB_TC_TMA2D=1)
-    if (freq && !(getenv("FCB_TC_TMA2D") && atoi(getenv("FCB_TC_TMA2D")) != 0)) want_raw = false;
+    // 2-D layers keep the per-thread gather: the K_F-fold re-read of every input row makes the unit stream L2-bound either way,
+    // and staging it through the raw ring measured slower at config 4 (r2g: conv stack 37.3 vs 33.6 ms)
+    bool want_raw = g_tma_state == 1 && !freq && (n_tt >= 3 || (p.K == 1 && p.S == 1 && p.pad_l == 0)) && p.T_in / p.S >= 1 &&
+                    (p.C_in % TC_KC == 0 || p.C_in == 16);
     TcPlan pl{};
     if (want_raw) {
-        pl = tc_plan(p, g_na_tma, true, g_deep_ring);
-        want_raw = pl.ok && pl.nraw >= 2;
-        if (want_raw && !freq)
-            want_raw = make_act_map(&tm0, p.in0, p.C_in, p.S, p.T_in, B, pl.L.a_rows) &&
-                       (!p.in1.x || make_act_map(&tm1, p.in1, p.C_in, p.S, p.T_in, B, pl.L.a_rows));
-        if (want_raw && freq) {
-            const int nclips = B / p.fq.F_out;
-            want_raw = make_act_map_2d(&tm0, p.in0, p.fq.cin, p.S, p.T_in, p.fq.F_in, p.fq.T_raw0, p.fq.f_off0, nclips, pl.L.a_rows) &&
-                       (!p.in1.x || make_act_map_2d(&tm1, p.in1, p.fq.cin, p.S, p.T_in, p.fq.F_in, p.fq.T_raw1, p.fq.f_off1, nclips, pl.L.a_rows));
-        }
+        pl = tc_plan(p, 2, true);
+        want_raw = pl.ok && pl.nraw >= 2 && make_act_map(&tm0, p.in0, p.C_in, p.S, p.T_in, B, pl.L.a_rows) &&
+                   (!p.in1.x || make_act_map(&tm1, p.in1, p.C_in, p.S, p.T_in, B, pl.L.a_rows));
     }
     if (!want_raw) {
-        pl = tc_plan(p, 4, false, g_deep_ring);
+        pl = tc_plan(p, 4, false);
         if (!pl.ok) return cudaErrorInvalidConfiguration;
     }
     switch (p.n_tile) {

@@ -82,14 +82,10 @@ struct fcb_handle {
     float* embed_tc = nullptr; // tensor-core image of the codebooks (rvq_tc.cu)
     int* err_flag = nullptr;
     unsigned* lstm_barrier = nullptr;
-    int* fin_counter = nullptr;  // per-clip partial counters of the fused GroupNorm finalisation (conv_tc.cu), zero between launches
     int rvq_sliced = 1;          // "rvq_sliced" option / FCB_RVQ_SLICED: the column-sliced fp32 RVQ kernel (rvq_simt.cu) for D > 260 (the
                                  // SoundStream YAMLs' D = 512; r2o found that such a D never fit the whole-chunk kernel).  Validated on
                                  // hardware in r2q (profiles/soundstream_fullwidth_r2q.txt: codes exact on 4 x 300 frames x 32 stages);
                                  // 0 makes fcb_finalize refuse such a D instead
-    int fuse_stats = 0;          // "fuse_stats" option / FCB_FUSE_STATS=1: GroupNorm finalisation inside the conv kernel.  OFF by default:
-                                 // measured slower at config 2 (r2m: conv stack 11.7 vs 10.8 ms -- the last CTA's serial reduction sits in
-                                 // every launch's tail) and neutral at B = 1; parity-tested, kept as an option
     unsigned long long* lstm_trace = nullptr;   // PROFILING ONLY (env FCB_LSTM_TRACE): managed buffer, dumped by fcb_destroy
     bool use_tc = true;      // tensor-core conv path (FCB_DISABLE_TC=1 or fcb_set_option disables it)
     int use_tc2d = 7;        // FreqCodec 2-D layers on the tensor-core path, bit mask of Conv2W::tc_class ("use_tc2d" option)
@@ -548,11 +544,6 @@ int run_conv(Run& r, const Act& in0, const Act* in1, bool elu, const float* div_
         o.gamma = L.gamma; o.beta = L.beta;
     }
     p.partials = partials;
-    const bool fused = tc && want_norm && h->fuse_stats && r.B <= 1024;
-    if (fused) {     // the conv kernel's last CTA per clip finalises the statistics itself
-        p.fin_counter = h->fin_counter; p.fin_stats = o.stats; p.fin_coef = o.coef; p.fin_gamma = L.gamma; p.fin_beta = L.beta;
-        p.fin_C = o.C; p.fin_parts = nparts; p.fin_count = (double)p.T_out * p.C_out; p.fin_eps = h->cfg.gn_eps;
-    }
     int np2 = 0;
     if (tc) FCB_CK(launch_conv_tc(p, r.B, r.st, &np2));
     else if (c1) FCB_CK(launch_conv_cout1(p, r.B, r.st, &np2));
@@ -560,11 +551,9 @@ int run_conv(Run& r, const Act& in0, const Act* in1, bool elu, const float* div_
     h->launches++;
     if (want_norm) {
         if (np2 != nparts) return fail(h, FCB_E_INVALID, "internal: partial count mismatch");
-        if (!fused) {
-            FCB_CK(launch_stats_finalize(partials, nparts, (double)p.T_out * p.C_out, h->cfg.gn_eps, 0, o.stats, r.B, r.st,
-                                         L.gamma, L.beta, o.C, o.coef));
-            h->launches++;
-        }
+        FCB_CK(launch_stats_finalize(partials, nparts, (double)p.T_out * p.C_out, h->cfg.gn_eps, 0, o.stats, r.B, r.st,
+                                     L.gamma, L.beta, o.C, o.coef));
+        h->launches++;
         FCB_TRY(pool_free(r, partials));
     }
     *out = o;
@@ -933,7 +922,6 @@ int run_conv2d(Run& r, const Act2& in0, const Act2* in1, bool elu, const Conv2W&
     FCB_TRY(alloc_f(r, &o.coef, (size_t)r.B * 2 * o.C));
     o.gamma = L.gamma; o.beta = L.beta;
     p.partials = partials;
-    bool fused2 = false;
     if (tc) {
         ConvParams q{};
         q.in0.x = in0.p; q.in0.coef = in0.coef; q.in0.row_off = in0.t_off;
@@ -955,11 +943,6 @@ int run_conv2d(Run& r, const Act2& in0, const Act2* in1, bool elu, const Conv2W&
         q.fq.FR = p.FR; q.fq.TR = p.TR;
         q.fq.Cc = L.tc_class == 4 ? L.cout_tc : p.Cc;      // padded image: one phase of cout_tc columns, Cc real ones stored
         q.fq.c_store = p.Cc;
-        fused2 = h->fuse_stats && r.B <= 1024;
-        if (fused2) {
-            q.fin_counter = h->fin_counter; q.fin_stats = o.stats; q.fin_coef = o.coef; q.fin_gamma = L.gamma; q.fin_beta = L.beta;
-            q.fin_C = o.C; q.fin_parts = nparts; q.fin_count = (double)per_clip; q.fin_eps = h->cfg.gn_eps;
-        }
         int np2 = 0;
         FCB_CK(launch_conv_tc(q, r.B * p.F_out, r.st, &np2));
         if (np2 * p.F_out != nparts) return fail(h, FCB_E_INVALID, "internal: partial count mismatch (2-D)");
@@ -968,10 +951,9 @@ int run_conv2d(Run& r, const Act2& in0, const Act2* in1, bool elu, const Conv2W&
     } else {
         FCB_CK(launch_conv2d(p, r.st));
     }
-    if (!fused2)
-        FCB_CK(launch_stats_finalize(partials, nparts, (double)per_clip, h->cfg.gn_eps, 0, o.stats, r.B, r.st, L.gamma,
-                                     L.beta, o.C, o.coef));
-    h->launches += fused2 ? 1 : 2;
+    FCB_CK(launch_stats_finalize(partials, nparts, (double)per_clip, h->cfg.gn_eps, 0, o.stats, r.B, r.st, L.gamma,
+                                 L.beta, o.C, o.coef));
+    h->launches += 2;
     FCB_TRY(pool_free(r, partials));
     *out = o;
     return FCB_OK;
@@ -1445,10 +1427,6 @@ int fcb_finalize(fcb_handle* h) {
     FCB_CK(cudaMemset(h->err_flag, 0, sizeof(int)));
     FCB_CK(cudaMalloc((void**)&h->lstm_barrier, 64 * sizeof(unsigned)));
     h->dev_allocs.push_back(h->lstm_barrier);
-    FCB_CK(cudaMalloc((void**)&h->fin_counter, 1024 * sizeof(int)));
-    FCB_CK(cudaMemset(h->fin_counter, 0, 1024 * sizeof(int)));
-    h->dev_allocs.push_back(h->fin_counter);
-    if (const char* v = getenv("FCB_FUSE_STATS")) h->fuse_stats = atoi(v) != 0;
     if (getenv("FCB_LSTM_TRACE")) {
         FCB_CK(cudaMallocManaged((void**)&h->lstm_trace, LSTM_TRACE_ITEMS * 8 * sizeof(unsigned long long)));
         FCB_CK(cudaMemset(h->lstm_trace, 0, LSTM_TRACE_ITEMS * 8 * sizeof(unsigned long long)));
@@ -1783,10 +1761,6 @@ int fcb_set_option(fcb_handle* h, const char* key, int32_t value) {
     if (strcmp(key, "rvq_sliced") == 0) {          // column-sliced fp32 RVQ kernel for D > 260 (default on; 0: refuse such a D)
         if (h->finalized) return fail(h, FCB_E_STATE, "rvq_sliced must be set before fcb_finalize");
         h->rvq_sliced = value != 0;
-        return FCB_OK;
-    }
-    if (strcmp(key, "fuse_stats") == 0) {          // GroupNorm finalisation inside the conv kernel vs a separate launch (default)
-        h->fuse_stats = value != 0;
         return FCB_OK;
     }
     if (strcmp(key, "conv2d_small_cout") == 0) {   // halo-tile SIMT kernel (default) vs the padded tensor-core n-tile

@@ -58,7 +58,6 @@ struct LstmSeqParams {
     InView skip;          // the SLSTM input (normalised on load) when y_out != nullptr
     unsigned* barrier;    // device counter for the per-step grid barrier (zeroed by the launcher)
     int B, T, H;
-    int fast_cell;        // hardware ex2 / rcp gates instead of expf / tanhf (set by the launcher: default 1, FCB_LSTM_FASTCELL=0 disables)
     float whh_scale, whh_inv_scale;   // tensor-core gate GEMM: power-of-two operand scale of W_hh and 1 / (whh_scale * 4096) (0: fp32 path)
     unsigned long long* trace;   // PROFILING ONLY (env FCB_LSTM_TRACE): [LSTM_TRACE_ITEMS][8] %globaltimer stamps of CTA 0, or nullptr
 };

@@ -18,7 +18,6 @@
 // Latency-bound by construction (T' dependent steps); FLOPs = 2*B*T*4H*H per layer.
 #include <cooperative_groups.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -26,17 +25,19 @@
 
 namespace fcb {
 
-constexpr int LSTM_GB_MAX = 8;    // clips per work item (accumulator tile): 8, or 4 for small batches (more items in flight)
+// clips per work item (accumulator tile).  4-clip groups (4 independent chains for B = 16) were measured twice: on the 2-slot
+// ring of round 1 (no gain) and with one ring slot per group (r2d: 3.67 vs 3.32 ms per SLSTM at config 2) -- the per-item
+// fixed costs (poll, bulk copy, reduction, publish) outweigh the shorter gate GEMM.
+constexpr int LSTM_GB = 8;
 constexpr int LSTM_NBUF_MAX = 8;  // h ring depth: 2 .. 8 slots, as many as shared memory holds (more independent clip groups in flight)
 constexpr int LSTM_THREADS = 480; // 8 compute warps, up to 3 x 2 cell warps (items round-robin), 1 loader warp: 15 warps keep the
                                   // 128-register budget of the 16-warp allocation bucket (17 warps drop to 96: measured slower)
 constexpr int LSTM_PAIRS_MAX = 3;
 constexpr int LSTM_MAX_GROUPS = 64;
 
-__device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
-// Gates on the hardware ex2 / rcp units (default; FCB_LSTM_FASTCELL=0 selects expf / tanhf): ~3e-7 relative instead of ~1e-7, a
-// much shorter dependent chain in the cell phase that heads every timestep's critical path.  Measured (r2fc): 17.73 -> 17.44 ms
-// per config-2 step with an IDENTICAL parity table (same 3999 / 4000 frames, waveforms 1.2e-6).
+// Gates on the hardware ex2 / rcp units: ~3e-7 relative instead of ~1e-7 for expf / tanhf, a much shorter dependent chain in
+// the cell phase that heads every timestep's critical path.  Measured (r2fc): 17.73 -> 17.44 ms per config-2 step with an
+// IDENTICAL parity table (same 3999 / 4000 frames, waveforms 1.2e-6).
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float sigmoid_fast(float x) { return rcp_approx(1.0f + tc::exp2f_approx(-1.4426950408889634f * x)); }
 __device__ __forceinline__ float tanh_fast(float x) { return fmaf(-2.0f, rcp_approx(1.0f + tc::exp2f_approx(2.8853900817779268f * x)), 1.0f); }
@@ -84,8 +85,9 @@ constexpr float LSTM_H_SCALE = 4096.0f;   // |h| < 1: fp16 operand scale of the 
 // lo*hi + hi*lo + hi*hi in fp32, exact inverse scale afterwards): ~2^-22 relative like the fp32 FMA chain it replaces, at a
 // third of the shared-memory instruction count -- the item then costs one pass over the 128 KB W_hh slice (LDS-bound).
 // The W slice lives in shared memory in FRAGMENT ORDER: [k-step (16 k)][m-tile (16 columns)][hi | lo][lane][8 halfs].
-template <int UNITS, int GB, bool MMA>
+template <int UNITS, bool MMA>
 __global__ void __launch_bounds__(LSTM_THREADS, 1) lstm_seq_kernel(const LstmSeqParams p, const int nbuf, const int npair, const int pload, const int nset) {
+    constexpr int GB = LSTM_GB;
     constexpr int COLS = 4 * UNITS;            // gate columns owned by this CTA
     constexpr int KS_PER_WARP = 32 / UNITS;    // K slices inside a warp
     // compute-warp sets: nset = 1: all 8 warps split the K dimension of one item; nset = 2 (narrow layers, where an item is bound
@@ -331,13 +333,11 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) lstm_seq_kernel(const LstmSeq
             long long o = 0;
             if (mine) {
                 const int b = b0 + fbb, j = j0 + fu;
-                float ig, fg, gg, og;
-                if (p.fast_cell) { ig = sigmoid_fast(g4[0]); fg = sigmoid_fast(g4[1]); gg = tanh_fast(g4[2]); og = sigmoid_fast(g4[3]); }
-                else { ig = sigmoidf_(g4[0]); fg = sigmoidf_(g4[1]); gg = tanhf(g4[2]); og = sigmoidf_(g4[3]); }
+                const float ig = sigmoid_fast(g4[0]), fg = sigmoid_fast(g4[1]), gg = tanh_fast(g4[2]), og = sigmoid_fast(g4[3]);
                 float* cp = cS + (g * GB + fbb) * UNITS + fu;
                 const float c = fg * (*cp) + ig * gg;
                 *cp = c;
-                h = og * (p.fast_cell ? tanh_fast(c) : tanhf(c));
+                h = og * tanh_fast(c);
                 o = ((long long)b * T + t) * H + j;
                 __stcg(p.h_seq + o, h);
             }
@@ -401,7 +401,8 @@ __global__ void __launch_bounds__(LSTM_THREADS, 1) lstm_seq_kernel(const LstmSeq
     }
 }
 
-size_t lstm_seq_smem_bytes(int H, int B, int units, int gb, int nbuf = 2, int npair = 2, bool ring = true) {
+size_t lstm_seq_smem_bytes(int H, int B, int units, int nbuf = 2, int npair = 2, bool ring = true) {
+    constexpr int gb = LSTM_GB;
     const int ng = (B + gb - 1) / gb;
     const size_t cs = ((size_t)ng * gb * units + 3) & ~(size_t)3;
     return ((size_t)H * 4 * units + (ring ? (size_t)nbuf * gb * H : 0) + (size_t)npair * 8 * 4 * units * gb + cs) * sizeof(float) +
@@ -410,34 +411,24 @@ size_t lstm_seq_smem_bytes(int H, int B, int units, int gb, int nbuf = 2, int np
 
 // h ring depth: one slot per independent clip group (their barrier / broadcast latencies overlap), 2 .. LSTM_NBUF_MAX,
 // limited by shared memory (H = 1024: the 128 KB W_hh slice leaves room for 2 slots of 32 KB)
-static int lstm_pick_nbuf(int H, int B, int units, int gb, bool ring) {
-    const int ng = (B + gb - 1) / gb;
+static int lstm_pick_nbuf(int H, int B, int units, bool ring) {
+    const int ng = (B + LSTM_GB - 1) / LSTM_GB;
     int nbuf = ng < 2 ? 2 : (ng > LSTM_NBUF_MAX ? LSTM_NBUF_MAX : ng);
-    while (nbuf > 2 && lstm_seq_smem_bytes(H, B, units, gb, nbuf, 2, ring) > 220 * 1024) --nbuf;
-    if (const char* v = getenv("FCB_LSTM_NBUF")) { const int f = atoi(v); if (f >= 2 && f <= nbuf) nbuf = f; }   // experiments
+    while (nbuf > 2 && lstm_seq_smem_bytes(H, B, units, nbuf, 2, ring) > 220 * 1024) --nbuf;
     return nbuf;
-}
-
-// clip-group size: 8 clips per work item.  4-clip groups (4 independent chains for B = 16) were measured twice: on the 2-slot
-// ring of round 1 (no gain) and with one ring slot per group (r2d: 3.67 vs 3.32 ms per SLSTM at config 2) -- the per-item
-// fixed costs (poll, bulk copy, reduction, publish) outweigh the shorter gate GEMM.
-static int lstm_pick_gb(int B) {
-    (void)B;
-    int gb = 8;
-    if (const char* v = getenv("FCB_LSTM_GB")) { const int f = atoi(v); if (f == 4 || f == 8) gb = f; }   // experiments
-    return gb;
 }
 
 int lstm_pick_units(int H) {
     // largest slice that fits shared memory while keeping >= 96 CTAs busy when H allows it
-    if (H % 8 == 0 && lstm_seq_smem_bytes(H, 16, 8, LSTM_GB_MAX) <= 220 * 1024 && H / 8 >= 96) return 8;
-    if (H % 4 == 0 && lstm_seq_smem_bytes(H, 16, 4, LSTM_GB_MAX) <= 220 * 1024) return 4;
+    if (H % 8 == 0 && lstm_seq_smem_bytes(H, 16, 8) <= 220 * 1024 && H / 8 >= 96) return 8;
+    if (H % 4 == 0 && lstm_seq_smem_bytes(H, 16, 4) <= 220 * 1024) return 4;
     return 0;
 }
 
-template <int UNITS, int GB, bool MMA>
+template <int UNITS, bool MMA>
 static cudaError_t launch_seq(const LstmSeqParams& p, cudaStream_t st) {
-    int nbuf = lstm_pick_nbuf(p.H, p.B, UNITS, GB, true);
+    constexpr int GB = LSTM_GB;
+    int nbuf = lstm_pick_nbuf(p.H, p.B, UNITS, true);
     // cell pairs: 3 when there are at least 3 independent clip groups to keep busy and the extra exchange buffer fits
     // per-group loader lanes only pay with many groups (r2f / r2g: config 2 (2 groups) 3.7 vs 3.45 ms, config 4 (4 groups) 8.15 vs
     // 6.5 ms, config 3 (8 groups) 36.8 vs 38.0 ms per SLSTM)
@@ -445,14 +436,11 @@ static cudaError_t launch_seq(const LstmSeqParams& p, cudaStream_t st) {
     int npair = 2, pload = ngroups >= 8 ? 1 : 0;
     // two compute-warp sets when an item's gate GEMM is small (H <= 512) and there are other groups to work on
     int nset = (p.H <= 512 && ngroups >= 2) ? 2 : 1;
-    if (const char* v = getenv("FCB_LSTM_NSET")) { const int f = atoi(v); if (f == 1 || f == 2) nset = f; }                // experiments
-    if ((p.B + GB - 1) / GB >= 3 && lstm_seq_smem_bytes(p.H, p.B, UNITS, GB, nbuf, 3) <= 220 * 1024) npair = 3;
-    if (const char* v = getenv("FCB_LSTM_PAIRS")) { const int f = atoi(v); if (f == 2 || (f == 3 && npair == 3)) npair = f; }   // experiments
-    if (const char* v = getenv("FCB_LSTM_PLOAD")) pload = atoi(v) != 0;
-    const size_t smem = lstm_seq_smem_bytes(p.H, p.B, UNITS, GB, nbuf, npair);
+    if ((p.B + GB - 1) / GB >= 3 && lstm_seq_smem_bytes(p.H, p.B, UNITS, nbuf, 3) <= 220 * 1024) npair = 3;
+    const size_t smem = lstm_seq_smem_bytes(p.H, p.B, UNITS, nbuf, npair);
     // the tensor-core gate GEMM needs whole k-steps per warp
-    if (MMA && (p.H % 16 != 0 || ((p.H / 16) % (8 / nset)) != 0 || (p.H / 16) / (8 / nset) > 8)) return launch_seq<UNITS, GB, false>(p, st);
-    auto kern = lstm_seq_kernel<UNITS, GB, MMA>;
+    if (MMA && (p.H % 16 != 0 || ((p.H / 16) % (8 / nset)) != 0 || (p.H / 16) / (8 / nset) > 8)) return launch_seq<UNITS, false>(p, st);
+    auto kern = lstm_seq_kernel<UNITS, MMA>;
     {
         cudaError_t e = ensure_dynamic_smem((const void*)kern, 225 * 1024);
         if (e != cudaSuccess) return e;
@@ -463,8 +451,6 @@ static cudaError_t launch_seq(const LstmSeqParams& p, cudaStream_t st) {
     if (e != cudaSuccess) return e;
     dim3 grid(p.H / UNITS), block(LSTM_THREADS);
     LstmSeqParams pc = p;
-    pc.fast_cell = 1;
-    if (const char* v = getenv("FCB_LSTM_FASTCELL")) pc.fast_cell = atoi(v) != 0;
     void* args[] = {&pc, &nbuf, &npair, &pload, &nset};
     return cudaLaunchCooperativeKernel((void*)kern, grid, block, args, smem, st);
 }
@@ -472,13 +458,9 @@ static cudaError_t launch_seq(const LstmSeqParams& p, cudaStream_t st) {
 cudaError_t launch_lstm_seq(const LstmSeqParams& p, cudaStream_t st) {
     if (p.H % 4 != 0) return cudaErrorInvalidValue;
     const int units = lstm_pick_units(p.H);
-    const int gb = lstm_pick_gb(p.B);
-    bool mma = p.whh_scale > 0.f;                     // tensor-core gate GEMM (default); FCB_LSTM_MMA=0: the fp32 FFMA2 path
-    if (const char* v = getenv("FCB_LSTM_MMA")) mma = mma && atoi(v) != 0;
-    if (units == 8 && gb == 8) return mma ? launch_seq<8, 8, true>(p, st) : launch_seq<8, 8, false>(p, st);
-    if (units == 8 && gb == 4) return launch_seq<8, 4, false>(p, st);
-    if (units == 4 && gb == 8) return mma ? launch_seq<4, 8, true>(p, st) : launch_seq<4, 8, false>(p, st);
-    if (units == 4 && gb == 4) return launch_seq<4, 4, false>(p, st);
+    const bool mma = p.whh_scale > 0.f;               // tensor-core gate GEMM; whh_scale == 0: the fp32 FFMA2 path
+    if (units == 8) return mma ? launch_seq<8, true>(p, st) : launch_seq<8, false>(p, st);
+    if (units == 4) return mma ? launch_seq<4, true>(p, st) : launch_seq<4, false>(p, st);
     return cudaErrorInvalidConfiguration;
 }
 

@@ -67,14 +67,6 @@ __device__ __forceinline__ void tma_load_4d(void* dst_smem, const void* tmap, in
         : "memory");
 }
 
-__device__ __forceinline__ void tma_load_5d(void* dst_smem, const void* tmap, int c0, int c1, int c2, int c3, int c4, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(
-            smem_u32(dst_smem)),
-        "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-        : "memory");
-}
-
 // ------------------------------------------------------------------------------------------------ tcgen05
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {   // one full warp; ncols pow2 >= 32
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
