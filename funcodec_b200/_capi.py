@@ -23,7 +23,7 @@ class FcbConfig(Structure):
                 ("gn_eps", c_float), ("arch", c_int32), ("ratios_f", c_int32 * FCB_MAX_RATIOS), ("n_fft", c_int32),
                 ("stft_hop", c_int32), ("conv_group_ratio", c_int32), ("tr_conv_group_ratio", c_int32),
                 ("n_residual_layers", c_int32), ("dilation_base", c_int32),
-                ("norm", c_int32), ("causal", c_int32)]
+                ("norm", c_int32), ("causal", c_int32), ("channels", c_int32)]
 
 
 FCB_MAX_TAIL_SEGMENTS = 16

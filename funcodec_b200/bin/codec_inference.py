@@ -82,6 +82,9 @@ def config_from_yaml(path: str):
     if enc.get("ratios", [8, 5, 4, 2]) != ratios:
         refuse("encoder and decoder ratios differ")
     domain = m.get("codec_domain", None)
+    # audio channels: top-level input_size feeds SEANetEncoder(input_size=...) and decoder_conf.channels the decoder's last
+    # conv (gan_speech_codec.py:304-329); the reference Encodec takes 1 or 2 (codec_basic.py:342-344)
+    channels = int(a.get("input_size", 1) or 1)
     kw = {}
     if a.get("model", "encodec") == "freq_codec" or (ratios and isinstance(ratios[0], (list, tuple))):
         if list(domain or []) != ["mag_phase", "mag_phase"]:
@@ -97,8 +100,14 @@ def config_from_yaml(path: str):
             refuse("segment_dur must be null for FreqCodec")
         if enc.get("norm", "weight_norm") != "time_group_norm" or enc.get("causal", False):
             refuse("FreqCodec: norm must be time_group_norm and causal false")
+        channels = 1          # input_size there counts the spectral features of the 2-D stacks; the waveform is mono
     elif domain not in (None, "time", ["time", "time"]):
         refuse(f"codec_domain {domain}")
+    else:
+        if int(dec.get("channels", 1)) != channels:
+            refuse(f"input_size {channels} != decoder_conf.channels {dec.get('channels', 1)}")
+        if channels not in (1, 2):
+            refuse(f"input_size {channels}: mono or stereo only")
     cfg = CodecConfig(name="from_yaml", ratios=tuple(int(r) for r in ratios), n_filters=int(enc.get("n_filters", 32)),
                       dimension=int(m.get("odim", 128)), kernel_size=int(enc.get("kernel_size", 7)),
                       last_kernel_size=int(enc.get("last_kernel_size", 7)),
@@ -110,7 +119,7 @@ def config_from_yaml(path: str):
                       # with one residual block the dilation base never shows (base ** 0 == 1): keep the default so that equal
                       # models compare equal
                       dilation_base=int(enc.get("dilation_base", 2)) if int(enc.get("n_residual_layers", 1)) > 1 else 2,
-                      norm=str(enc.get("norm", "weight_norm")), causal=bool(enc.get("causal", False)), **kw)
+                      norm=str(enc.get("norm", "weight_norm")), causal=bool(enc.get("causal", False)), channels=channels, **kw)
     if int(q.get("encoder_hop_length", cfg.hop_length)) != cfg.hop_length:
         refuse("quantizer_conf.encoder_hop_length != hop of the ratios")
     return cfg, m.get("segment_dur"), m.get("overlap_ratio")
@@ -172,9 +181,18 @@ def stat_flops_line(cfg: CodecConfig, bit_width=None) -> str:
             f"(conv {w['conv_macs'] / 1e9:.2f}G, LSTM {w['lstm_macs'] / 1e9:.2f}G, RVQ@{n_q} {w['rvq_flops'] / 2e9:.2f}G)")
 
 
+def refuse_stereo_file_io(cfg: CodecConfig):
+    """The file I/O here (wav.scp / PCM16 wav, one channel per utterance) is mono; the reference CLI cannot feed a stereo model
+    either (its [B, L, C] batches fail _encode's channel assert).  Stereo models run through B200Encodec with [B, 2, L] tensors."""
+    if cfg.channels != 1:
+        raise SystemExit(f"unsupported configuration: input_size {cfg.channels} (stereo) through the CLI's mono file I/O; "
+                         "call funcodec_b200.B200Encodec.inference with [B, 2, L] tensors instead")
+
+
 def build_speech2token(config_file: str, model_file: str, device: str = "cuda:0", need_sub_quants: bool = False):
     """`Speech2Token.from_pretrained` without the hub (codec_inference.py:136-150): YAML + checkpoint -> Speech2Token on B200Encodec."""
     cfg, segment_dur, overlap_ratio = config_from_yaml(config_file)
+    refuse_stereo_file_io(cfg)
     sd = torch.load(model_file, map_location="cpu")
     if isinstance(sd, dict) and "state_dict" in sd and not any(k.startswith("encoder.") for k in sd):
         sd = sd["state_dict"]
@@ -282,6 +300,7 @@ def main(argv=None):
     path, _name, dtype = args.data_path_and_name_and_type[0]
     device = f"cuda:{pick_gpu(args.output_dir, args.gpuid_list)}"
     cfg, segment_dur, overlap_ratio = config_from_yaml(args.config_file)
+    refuse_stereo_file_io(cfg)
     if cfg.sample_rate != args.sampling_rate:
         raise SystemExit(f"--sampling_rate {args.sampling_rate} != model rate {cfg.sample_rate}")
     if args.stat_flops:

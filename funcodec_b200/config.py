@@ -4,7 +4,7 @@ Mirrors the YAML keys the reference feeds to GANSpeechCodecTask.build_model
 (/root/reference/funcodec/tasks/gan_speech_codec.py:301-358): `encoder_conf`, `quantizer_conf`,
 `decoder_conf`, `model_conf` of egs/LibriTTS/codec/conf/encodec_16k_n32_600k_step{,_ds640}.yaml.
 Representable: norm time_group_norm / weight_norm / none, causal or not (time-domain stacks), true_skip=False, compress=2,
-LSTM or no sequence model, stacked dilated residual blocks, RVQ without projections.
+LSTM or no sequence model, stacked dilated residual blocks, RVQ without projections, mono or stereo time-domain audio.
 """
 from dataclasses import dataclass, field, asdict
 from typing import Dict, Optional, Tuple
@@ -44,6 +44,9 @@ class CodecConfig:
     # 'time_group_norm' | 'weight_norm' | 'none'; causal needs a norm other than time_group_norm (conv.py:46-47)
     norm: str = "time_group_norm"
     causal: bool = False
+    # audio channels of the time-domain stacks: top-level `input_size` / decoder_conf `channels` (seanet_encoder.py:91-110,
+    # seanet_decoder.py:89-161); 2 = stereo, waveforms [B, 2, L] (codec_basic.py:342-344 allows 1 or 2).  FreqCodec is mono.
+    channels: int = 1
 
     def conv_groups(self, channels: int) -> int:
         """groups of a 2-D conv whose reference expression is `channels // 2 // conv_group_ratio`."""
@@ -131,6 +134,16 @@ PRESETS: Dict[str, CodecConfig] = {
                                          codebook_size=64, num_quantizers=8, norm="weight_norm"),
     "small_ds320": CodecConfig(name="small_ds320", ratios=(8, 5, 4, 2), n_filters=8, dimension=64,
                                codebook_size=256, num_quantizers=8),
+    # the 48 kHz stereo layout seanet_encoder.py:63-65 names ("48HZ -> channels = 2, norm = time_group_norm, causal = False"):
+    # hop 320, 150 frames per second
+    "encodec_48k_stereo": CodecConfig(name="encodec_48k_stereo", ratios=(8, 5, 4, 2), sample_rate=48000, num_quantizers=16,
+                                      channels=2),
+    # small stereo shapes for the parity tests: time_group_norm + SLSTM, and weight_norm + causal (no GroupNorm on the last layer)
+    "stereo_small": CodecConfig(name="stereo_small", ratios=(5, 4, 2), n_filters=8, dimension=32, codebook_size=64,
+                                num_quantizers=8, channels=2),
+    "stereo_causal_small": CodecConfig(name="stereo_causal_small", ratios=(5, 4, 2), n_filters=4, dimension=48, codebook_size=64,
+                                       num_quantizers=4, lstm_layers=0, n_residual_layers=3, norm="weight_norm", causal=True,
+                                       channels=2),
 }
 
 

@@ -59,6 +59,8 @@ struct ConvParams {
     double* partials;        // [B][n_parts][2] (sum, sum of squares) or nullptr
     int cic;                 // input-channel chunk staged per iteration
     Freq2d fq;               // tensor-core 2-D mode (zero-initialised for 1-D layers)
+    long long in_ch_stride;  // 0: in0 is channels-last; else in0 is channel-planar [B][C_in][T_in] with this channel stride
+                             // (the stereo waveform [B, 2, L] read by the first encoder conv; SIMT kernel only)
 };
 
 // ---- FreqCodec 2-D path (conv2d_simt.cu): raw activations are channels-last [B][F_raw][T_raw][C]

@@ -96,7 +96,7 @@ __global__ void __launch_bounds__(256, TWO_LEVEL ? 1 : 2) conv1d_cl_kernel(const
                 if (p.pad_zero) ok = ok && gt >= 0 && gt < p.T_in;
                 else { src = reflect_index(gt, p.T_ext); ok = ok && src < p.T_in; }
                 if (ok) {
-                    const long long off = (long long)src * C_in + c;
+                    const long long off = p.in_ch_stride ? (long long)c * p.in_ch_stride + src : (long long)src * C_in + c;
                     float xv = __ldg(x0 + off);
                     if (p.div_scale) v = xv / inv_div;
                     else v = fmaf(xv, a0, b0);
@@ -235,18 +235,20 @@ __global__ void stats_finalize_kernel(const double* __restrict__ partials, int n
     }
 }
 
-// Per-clip sum of squares partials of the raw waveform (for the RMS scale).
+// Per-clip sum of squares partials of the raw waveform (for the RMS scale).  C = 2: the planar stereo clip [2][L]; the
+// squares are those of the mono mix m = (x0 + x1) * 0.5 rounded to fp32 first, as x.mean(dim=1) is (codec_basic.py:366-368).
+template <int C>
 __global__ void sumsq_partials_kernel(const float* __restrict__ x, int L, int chunk, double* __restrict__ partials) {
     __shared__ double red[64];
     const int b = blockIdx.y;
     const int start = blockIdx.x * chunk;
     const int end = min(L, start + chunk);
-    const float* xb = x + (long long)b * L;
+    const float* xb = x + (long long)b * C * L;
     float s = 0.f, ss = 0.f;
     double ds = 0.0, dss = 0.0;
     int n = 0;
     for (int i = start + threadIdx.x; i < end; i += blockDim.x) {
-        const float v = xb[i];
+        const float v = C == 1 ? xb[i] : __fmul_rn(__fadd_rn(xb[i], xb[(long long)(C - 1) * L + i]), 0.5f);
         s += v; ss = fmaf(v, v, ss);
         if (++n == 64) { ds += s; dss += ss; s = 0.f; ss = 0.f; n = 0; }
     }
@@ -258,19 +260,23 @@ __global__ void sumsq_partials_kernel(const float* __restrict__ x, int L, int ch
     }
 }
 
-// Conv with a single output channel (the decoder's last SConv1d, seanet_decoder.py:160-164): pure HBM streaming (reads C_in
-// floats per sample, writes one).  out[t] = bias + sum_k d_k[t + k - pad], d_k[r] = sum_c f(x[r][c]) w[k][c]: every input row is
-// loaded (coalesced: 8 lanes x 16 B per row, 4 rows per warp instruction), transformed and dotted with the K taps exactly ONCE
-// -- each lane holds the K x 4 weights of its 4 channels in registers, the 8 lanes of a row reduce with 3 shuffle levels -- and
-// the K partial products per row go through shared memory to the threads that own the outputs.  C_in == 32, K <= 8.
+// Conv with one or two output channels (the decoder's last SConv1d, seanet_decoder.py:160-164; CO = 2 for a stereo decoder):
+// pure HBM streaming (reads C_in floats per sample, writes CO).  out[t][co] = bias[co] + sum_k d_k,co[t + k - pad],
+// d_k,co[r] = sum_c f(x[r][c]) w[k][c][co]: every input row is loaded (coalesced: 8 lanes x 16 B per row, 4 rows per warp
+// instruction), transformed and dotted with the K x CO taps exactly ONCE -- each lane holds the K x 4 x CO weights of its 4
+// channels in registers, the 8 lanes of a row reduce with 3 shuffle levels -- and the K x CO partial products per row go
+// through shared memory to the threads that own the outputs.  The CTA's (sum, sum^2) covers all CO channels of its rows
+// (GroupNorm(1, CO), conv.py:45-52).  C_in == 32, K <= 8; the time tile shrinks with CO to keep the static shared memory.
 constexpr int C1_THREADS = 256, C1_TILE = 1024, C1_KMAX = 8;
 
+template <int CO>
 __global__ void __launch_bounds__(C1_THREADS) conv1d_cout1_kernel(const ConvParams p) {
-    __shared__ float D[C1_KMAX][C1_TILE + C1_KMAX];      // d_k of the tile's input rows (row index relative to t0 - pad_l)
+    constexpr int TILE = C1_TILE / CO;
+    __shared__ float D[CO][C1_KMAX][TILE + C1_KMAX];     // d_k,co of the tile's input rows (row index relative to t0 - pad_l)
     __shared__ double red[64];
     const int C_in = p.C_in, K = p.K;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, b = blockIdx.y;
-    const int t0 = blockIdx.x * C1_TILE;
+    const int t0 = blockIdx.x * TILE;
     const bool has1 = p.in1.x != nullptr;
     const int jchunk = lane & 7, rsub = lane >> 3;
     const int c = jchunk * 4;
@@ -285,11 +291,23 @@ __global__ void __launch_bounds__(C1_THREADS) conv1d_cout1_kernel(const ConvPara
         const float* cf = p.in1.coef + (long long)b * 2 * C_in;
         a1 = __ldg(reinterpret_cast<const float4*>(cf + c)); b1 = __ldg(reinterpret_cast<const float4*>(cf + C_in + c));
     }
-    float4 w[C1_KMAX];                                   // packed [k][ci][1]
+    float4 w[C1_KMAX][CO];                               // w[k][co] = taps of channels c..c+3 (packed [k][ci][co])
 #pragma unroll
-    for (int k = 0; k < C1_KMAX; ++k) w[k] = k < K ? __ldg(reinterpret_cast<const float4*>(p.w + k * C_in + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int k = 0; k < C1_KMAX; ++k) {
+        if (CO == 1) {
+            w[k][0] = k < K ? __ldg(reinterpret_cast<const float4*>(p.w + k * C_in + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        } else {
+            float4 lo = make_float4(0.f, 0.f, 0.f, 0.f), hi = lo;   // (c, co0) (c, co1) (c+1, co0) (c+1, co1) | c+2, c+3
+            if (k < K) {
+                lo = __ldg(reinterpret_cast<const float4*>(p.w + (k * C_in + c) * CO));
+                hi = __ldg(reinterpret_cast<const float4*>(p.w + (k * C_in + c) * CO + 4));
+            }
+            w[k][0] = make_float4(lo.x, lo.z, hi.x, hi.z);
+            w[k][CO - 1] = make_float4(lo.y, lo.w, hi.y, hi.w);
+        }
+    }
     const int gt_max = (p.T_out - 1) - p.pad_l + (K - 1);
-    const int R = min(C1_TILE, p.T_out - t0) + K - 1;   // input rows of this tile
+    const int R = min(TILE, p.T_out - t0) + K - 1;      // input rows of this tile
     constexpr int UNR = 4;                               // rows in flight per lane
     for (int rbase = warp * 4; rbase < R; rbase += 8 * 4 * UNR) {      // warp-uniform trip count (full-mask shuffles inside)
         const int r0 = rbase + rsub;
@@ -321,31 +339,47 @@ __global__ void __launch_bounds__(C1_THREADS) conv1d_cout1_kernel(const ConvPara
                 }
                 if (p.elu) { v.x = elu1(v.x); v.y = elu1(v.y); v.z = elu1(v.z); v.w = elu1(v.w); }
             }
-            float mine = 0.f;
+            float mine[CO];
+#pragma unroll
+            for (int co = 0; co < CO; ++co) mine[co] = 0.f;
 #pragma unroll
             for (int k = 0; k < C1_KMAX; ++k) {
-                float d = fmaf(v.w, w[k].w, fmaf(v.z, w[k].z, fmaf(v.y, w[k].y, v.x * w[k].x)));
-                d += __shfl_xor_sync(0xffffffffu, d, 1);
-                d += __shfl_xor_sync(0xffffffffu, d, 2);
-                d += __shfl_xor_sync(0xffffffffu, d, 4);
-                if (jchunk == k) mine = d;
+#pragma unroll
+                for (int co = 0; co < CO; ++co) {
+                    const float4 wk = w[k][co];
+                    float d = fmaf(v.w, wk.w, fmaf(v.z, wk.z, fmaf(v.y, wk.y, v.x * wk.x)));
+                    d += __shfl_xor_sync(0xffffffffu, d, 1);
+                    d += __shfl_xor_sync(0xffffffffu, d, 2);
+                    d += __shfl_xor_sync(0xffffffffu, d, 4);
+                    if (jchunk == k) mine[co] = d;
+                }
             }
-            if (row < R && jchunk < K) D[jchunk][row] = mine;
+            if (row < R && jchunk < K) {
+#pragma unroll
+                for (int co = 0; co < CO; ++co) D[co][jchunk][row] = mine[co];
+            }
         }
     }
     __syncthreads();
-    const float bias = __ldg(p.bias);
+    float bias[CO];
+#pragma unroll
+    for (int co = 0; co < CO; ++co) bias[co] = __ldg(p.bias + co);
     float s = 0.f, ss = 0.f;
     float* outb = p.out + (long long)b * p.out_clip_stride;
 #pragma unroll
-    for (int i = 0; i < C1_TILE / C1_THREADS; ++i) {
+    for (int i = 0; i < TILE / C1_THREADS; ++i) {
         const int tl = tid + C1_THREADS * i, t = t0 + tl;
         if (t < p.T_out) {
-            float acc = 0.f;
-            for (int k = 0; k < K; ++k) acc += D[k][tl + k];
-            const float o = acc + bias;
-            outb[t] = o;
-            s += o; ss = fmaf(o, o, ss);
+            float o[CO];
+#pragma unroll
+            for (int co = 0; co < CO; ++co) {
+                float acc = 0.f;
+                for (int k = 0; k < K; ++k) acc += D[co][k][tl + k];
+                o[co] = acc + bias[co];
+                s += o[co]; ss = fmaf(o[co], o[co], ss);
+            }
+            if (CO == 1) outb[t] = o[0];
+            else *reinterpret_cast<float2*>(outb + (long long)t * CO) = make_float2(o[0], o[CO - 1]);
         }
     }
     if (p.partials) {
@@ -359,15 +393,19 @@ __global__ void __launch_bounds__(C1_THREADS) conv1d_cout1_kernel(const ConvPara
 }
 
 bool conv_cout1_supported(const ConvParams& p) {
-    return p.C_out == 1 && p.S == 1 && p.D == 1 && !p.pad_zero && !p.div_scale && p.C_in == 32 && p.K <= C1_KMAX &&
-           !(p.in0.stats && !p.in0.coef) && !(p.in1.x && p.in1.stats && !p.in1.coef);
+    return (p.C_out == 1 || p.C_out == 2) && p.S == 1 && p.D == 1 && !p.pad_zero && !p.div_scale && !p.in_ch_stride &&
+           p.C_in == 32 && p.K <= C1_KMAX && !(p.in0.stats && !p.in0.coef) && !(p.in1.x && p.in1.stats && !p.in1.coef);
 }
-int conv_cout1_num_parts(int T_out) { return (T_out + C1_TILE - 1) / C1_TILE; }
+int conv_cout1_num_parts(int T_out, int C_out) {
+    const int tile = C1_TILE / C_out;
+    return (T_out + tile - 1) / tile;
+}
 
 cudaError_t launch_conv_cout1(const ConvParams& p, int B, cudaStream_t st, int* nparts) {
-    dim3 grid(conv_cout1_num_parts(p.T_out), B);
+    dim3 grid(conv_cout1_num_parts(p.T_out, p.C_out), B);
     *nparts = grid.x;
-    conv1d_cout1_kernel<<<grid, C1_THREADS, 0, st>>>(p);
+    if (p.C_out == 2) conv1d_cout1_kernel<2><<<grid, C1_THREADS, 0, st>>>(p);
+    else conv1d_cout1_kernel<1><<<grid, C1_THREADS, 0, st>>>(p);
     return cudaGetLastError();
 }
 
@@ -436,11 +474,12 @@ cudaError_t launch_stats_finalize(const double* partials, int nparts, double cou
     return cudaGetLastError();
 }
 
-cudaError_t launch_sumsq_partials(const float* x, int B, int L, double* partials, int* nparts, cudaStream_t st) {
+cudaError_t launch_sumsq_partials(const float* x, int B, int L, double* partials, int* nparts, cudaStream_t st, int C) {
     const int chunk = 16384;
     const int n = (L + chunk - 1) / chunk;
     *nparts = n;
-    sumsq_partials_kernel<<<dim3(n, B), 256, 0, st>>>(x, L, chunk, partials);
+    if (C == 2) sumsq_partials_kernel<2><<<dim3(n, B), 256, 0, st>>>(x, L, chunk, partials);
+    else sumsq_partials_kernel<1><<<dim3(n, B), 256, 0, st>>>(x, L, chunk, partials);
     return cudaGetLastError();
 }
 

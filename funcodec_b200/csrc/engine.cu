@@ -61,6 +61,7 @@ struct Act {
     const float* gamma = nullptr;
     const float* beta = nullptr;
     bool owned = false;              // p (and stats) were allocated from the pool by the engine
+    long long ch_stride = 0;         // 0: channels-last; else channel-planar [B][C][T] (the stereo waveform), this channel stride
 };
 
 }  // namespace
@@ -125,6 +126,7 @@ struct fcb_handle {
     // samples per codec frame: prod(ratios), times the STFT hop for the FreqCodec variant
     int hop() const { return cfg.arch == 1 ? tprod() * cfg.stft_hop : tprod(); }
     int top_channels() const { return cfg.n_filters << cfg.n_ratios; }
+    int channels() const { return cfg.channels == 2 ? 2 : 1; }   // audio channels (fcb_config.channels 0 / 1: mono)
 };
 
 namespace {
@@ -498,6 +500,7 @@ int run_conv(Run& r, const Act& in0, const Act* in1, bool elu, const float* div_
     p.div_scale = div_scale;
     p.elu = elu ? 1 : 0;
     p.T_in = in0.T; p.C_in = in0.C;
+    p.in_ch_stride = in0.ch_stride;
     if (in0.C != L.cin) return fail(h, FCB_E_INVALID, "internal: channel mismatch");
     Act o;
     if (!L.transposed) {
@@ -529,14 +532,14 @@ int run_conv(Run& r, const Act& in0, const Act* in1, bool elu, const float* div_
     }
     p.w = L.w; p.bias = L.bias; p.w_tc = L.w_tc; p.n_tile = L.n_tile; p.tc_w_scale = L.tc_scale;
     p.out_clip_stride = (long long)p.T_out * p.C_out;
-    const bool tc = h->use_tc && L.n_tile > 0 && L.w_tc && !div_scale;
+    const bool tc = h->use_tc && L.n_tile > 0 && L.w_tc && !div_scale && !in0.ch_stride;
     FCB_TRY(alloc_f(r, &o.p, (size_t)r.B * p.out_clip_stride));
     o.owned = true;
     p.out = o.p;
     double* partials = nullptr;
     const bool c1 = !tc && conv_cout1_supported(p);
     const int nparts = tc ? conv_tc_num_parts(p.T_out, p.C_out)
-                          : (c1 ? conv_cout1_num_parts(p.T_out) : conv_num_parts(p.T_out, p.C_out, p.C_in, p.K, r.B));
+                          : (c1 ? conv_cout1_num_parts(p.T_out, p.C_out) : conv_num_parts(p.T_out, p.C_out, p.C_in, p.K, r.B));
     if (want_norm) {
         FCB_TRY(pool_alloc(r, (void**)&partials, (size_t)r.B * nparts * 2 * sizeof(double)));
         FCB_TRY(alloc_f(r, &o.stats, (size_t)r.B * 2));
@@ -612,10 +615,11 @@ int run_resblock(Run& r, const Act& x, const ResBlockW& W, Act* sc_out, Act* blk
 }
 
 // Encodec._encode_frame (codec_basic.py:361-380) + SEANetEncoder.forward; returns the final conv's raw
-// output view (GroupNorm deferred into the RVQ kernel's load).
+// output view (GroupNorm deferred into the RVQ kernel's load).  wav is [B][L], or channel-planar [B][2][L] for a stereo
+// handle: the scale comes from the mono mix and the first conv reads both channel rows directly.
 int run_encoder(Run& r, const float* wav, int L, float* scale_out, Act* out) {
     fcb_handle* h = r.h;
-    const int B = r.B;
+    const int B = r.B, C = h->channels();
     FCB_TRY(phase_begin(r, FCB_PHASE_ENCODER_CONV));
     float* scale = nullptr;
     bool scale_owned = false;
@@ -624,7 +628,7 @@ int run_encoder(Run& r, const float* wav, int L, float* scale_out, Act* out) {
         int nparts = sumsq_num_parts(L), np2 = 0;
         FCB_TRY(pool_alloc(r, (void**)&partials, (size_t)B * nparts * 2 * sizeof(double)));
         if (scale_out) scale = scale_out; else { FCB_TRY(alloc_f(r, &scale, B)); scale_owned = true; }
-        FCB_CK(launch_sumsq_partials(wav, B, L, partials, &np2, r.st));
+        FCB_CK(launch_sumsq_partials(wav, B, L, partials, &np2, r.st, C));
         FCB_CK(launch_stats_finalize(partials, nparts, (double)L, 0.f, 1, scale, B, r.st));
         h->launches += 2;
         FCB_TRY(pool_free(r, partials));
@@ -633,7 +637,8 @@ int run_encoder(Run& r, const float* wav, int L, float* scale_out, Act* out) {
         h->launches++;
     }
     Act x;
-    x.p = const_cast<float*>(wav); x.T = L; x.C = 1; x.clip_stride = L;
+    x.p = const_cast<float*>(wav); x.T = L; x.C = C; x.clip_stride = (long long)C * L;
+    if (C > 1) x.ch_stride = L;
     Act a;
     FCB_TRY(run_conv(r, x, nullptr, false, scale, h->enc_conv0, true, &a));
     if (scale_owned) FCB_TRY(pool_free(r, scale));
@@ -717,7 +722,7 @@ int run_decoder_time(Run& r, const float* emb, int n_frames, const float* scale,
     FCB_TRY(run_conv(r, sc, have_blk ? &blk : nullptr, true, nullptr, h->dec_final, true, &f));
     FCB_TRY(release(r, sc));
     if (have_blk) FCB_TRY(release(r, blk));
-    FCB_CK(launch_final_output(f.p, f.stats, f.gamma, f.beta, scale, r.B, f.T, out_len, wav_out, r.st));
+    FCB_CK(launch_final_output(f.p, f.stats, f.gamma, f.beta, scale, r.B, f.T, out_len, wav_out, r.st, f.C));
     h->launches++;
     FCB_TRY(release(r, f));
     FCB_TRY(phase_end(r));
@@ -1291,6 +1296,8 @@ int fcb_create(const fcb_config* cfg, fcb_handle** out) {
     if (cfg->norm < 0 || cfg->norm > 2 || (cfg->causal != 0 && cfg->causal != 1)) return FCB_E_INVALID;
     if (cfg->causal && cfg->norm == 0) return FCB_E_INVALID;      // "GroupNorm doesn't support causal evaluation" (conv.py:46-47)
     if (cfg->arch == 1 && (cfg->norm != 0 || cfg->causal)) return FCB_E_INVALID;   // FreqCodec: time_group_norm, non-causal only
+    if (cfg->channels < 0 || cfg->channels > 2) return FCB_E_INVALID;              // the reference asserts 0 < channels <= 2
+    if (cfg->arch == 1 && cfg->channels == 2) return FCB_E_INVALID;                // FreqCodec STFTs x.squeeze(1): mono only
     if (cfg->arch == 1) {
         if (cfg->n_fft < 16 || cfg->n_fft % 2 != 0 || cfg->stft_hop < 1 || cfg->stft_hop > cfg->n_fft) return FCB_E_INVALID;
         for (int i = 0; i < cfg->n_ratios; ++i)
@@ -1341,7 +1348,8 @@ int fcb_finalize(fcb_handle* h) {
     if (c.arch == 1) {
         FCB_TRY(finalize_freq(h));
     } else {
-    FCB_TRY(pack_conv(h, "encoder.model.0", 1, nf, c.kernel_size, 1, &h->enc_conv0));
+    const int ch = h->channels();
+    FCB_TRY(pack_conv(h, "encoder.model.0", ch, nf, c.kernel_size, 1, &h->enc_conv0));
     int n = 1, mult = 1;
     const int nres = c.n_residual_layers > 0 ? c.n_residual_layers : 1, dbase = c.dilation_base > 0 ? c.dilation_base : 2;
     for (int i = c.n_ratios - 1; i >= 0; --i) {      // encoder applies the ratios reversed (seanet_encoder.py:102)
@@ -1382,7 +1390,12 @@ int fcb_finalize(fcb_handle* h) {
         }
         mult /= 2; n += nres + 2;
     }
-    FCB_TRY(pack_conv(h, "decoder.model." + std::to_string(n + 1), nf, 1, c.last_kernel_size, 1, &h->dec_final));
+    FCB_TRY(pack_conv(h, "decoder.model." + std::to_string(n + 1), nf, ch, c.last_kernel_size, 1, &h->dec_final));
+    // the stereo layers need the SIMT kernels: the first conv reads the planar waveform, and the decoder output goes
+    // channels-last [T][2] into final_output_kernel; neither has a tensor-core form
+    if (ch > 1 && (h->enc_conv0.n_tile > 0 || h->dec_final.n_tile > 0))
+        return fail(h, FCB_E_INVALID, "stereo: the first encoder conv and the last decoder conv have no tensor-core path "
+                    "for 2 channels (planar input / C_out = 2)");
     }
 
     if (!find(h, "quantizer.rq.model.embed") && find(h, "quantizer.rq.model.layers.0._codebook.embed")) {
@@ -1639,11 +1652,12 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
     FCB_TRY(fcb_plan_segments(h, L, seg_len, stride, &pl));
     cudaStream_t st = (cudaStream_t)stream;
     const int D = h->cfg.dimension, hop = h->hop();
+    const int C = h->channels();           // a planar clip [C][L] is C rows for the gather and overlap-add kernels
     const bool apply = use_scale && h->cfg.audio_normalize;
     Run r{h, B, st};                       // owner of the temporaries that span the whole call
     OlaParams ola{};
     float* frames_full = nullptr;
-    if (recon && pl.n_full > 0) FCB_TRY(alloc_f(r, &frames_full, (size_t)pl.n_full * B * pl.decoded_full));
+    if (recon && pl.n_full > 0) FCB_TRY(alloc_f(r, &frames_full, (size_t)pl.n_full * B * C * pl.decoded_full));
     // ---- the full-length segments: one batch of n_full*B clips, in chunks of <= 512 clips
     const int n_clips = pl.n_full * B, T0 = pl.frames_full;
     for (int c0 = 0; c0 < n_clips; ) {
@@ -1655,8 +1669,8 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
         const int nc = segs * B;
         Run rc{h, nc, st};
         float* x = nullptr;
-        FCB_TRY(alloc_f(rc, &x, (size_t)nc * seg_len));
-        FCB_CK(launch_gather_segments(wav, B, L, seg_len, stride, s0, segs, x, st));
+        FCB_TRY(alloc_f(rc, &x, (size_t)nc * C * seg_len));
+        FCB_CK(launch_gather_segments(wav, B * C, L, seg_len, stride, s0, segs, x, st));
         h->launches++;
         float* q = quant ? quant + (size_t)c0 * T0 * D : nullptr;
         float* sc = scale ? scale + c0 : nullptr;
@@ -1670,7 +1684,7 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
         if (!whole)
             FCB_CK(cudaMemcpy2DAsync(cdst, (size_t)n_clips * T0 * sizeof(int64_t), ctmp, (size_t)nc * T0 * sizeof(int64_t),
                                      (size_t)nc * T0 * sizeof(int64_t), n_q, cudaMemcpyDeviceToDevice, st));
-        if (recon) FCB_TRY(run_decoder(rc, q, T0, apply ? sc : nullptr, frames_full + (size_t)c0 * pl.decoded_full, pl.decoded_full));
+        if (recon) FCB_TRY(run_decoder(rc, q, T0, apply ? sc : nullptr, frames_full + (size_t)c0 * C * pl.decoded_full, pl.decoded_full));
         c0 += nc;
     }
     // ---- the shorter trailing segments, one by one
@@ -1679,8 +1693,8 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
         const int len = pl.tail_len[i], Ti = pl.tail_frames[i], dl = Ti * hop;
         Run rc{h, B, st};
         float* x = nullptr;
-        FCB_TRY(alloc_f(rc, &x, (size_t)B * len));
-        FCB_CK(launch_gather_segments(wav, B, L, len, stride, pl.n_full + i, 1, x, st));
+        FCB_TRY(alloc_f(rc, &x, (size_t)B * C * len));
+        FCB_CK(launch_gather_segments(wav, B * C, L, len, stride, pl.n_full + i, 1, x, st));
         h->launches++;
         float* q = quant ? quant + quant_off : nullptr;
         float* sc = scale ? scale + (size_t)(pl.n_full + i) * B : nullptr;
@@ -1689,7 +1703,7 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
         FCB_TRY(do_encode(h, x, B, len, n_q, codes + code_off, q, sc, nullptr, nullptr, st));
         if (recon) {
             float* fr = nullptr;
-            FCB_TRY(alloc_f(r, &fr, (size_t)B * dl));
+            FCB_TRY(alloc_f(r, &fr, (size_t)B * C * dl));
             FCB_TRY(run_decoder(rc, q, Ti, apply ? sc : nullptr, fr, dl));
             ola.tail[i] = fr; ola.tail_dl[i] = dl;
         }
@@ -1699,7 +1713,7 @@ int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t 
     if (recon) {
         ola.full = frames_full; ola.n_seg = pl.n_seg; ola.n_full = pl.n_full;
         ola.dl0 = pl.n_full > 0 ? pl.decoded_full : ola.tail_dl[0];       // weights come from the FIRST frame's length
-        ola.stride = stride; ola.B = B; ola.out_len = L; ola.out = recon;
+        ola.stride = stride; ola.B = B * C; ola.out_len = L; ola.out = recon;
         FCB_CK(launch_overlap_add(ola, st));
         h->launches++;
     }
@@ -1714,16 +1728,17 @@ int fcb_roundtrip_host(fcb_handle* h, const float* wav_host, int32_t B, int32_t 
     cudaStream_t st = (cudaStream_t)stream;
     Run r{h, B, st};
     const int Tf = fcb_num_frames(h, L);
+    const size_t n_wav = (size_t)B * h->channels() * L;
     float *d_wav, *d_recon;
     int64_t* d_codes;
-    FCB_TRY(alloc_f(r, &d_wav, (size_t)B * L));
-    FCB_TRY(alloc_f(r, &d_recon, (size_t)B * L));
+    FCB_TRY(alloc_f(r, &d_wav, n_wav));
+    FCB_TRY(alloc_f(r, &d_recon, n_wav));
     FCB_TRY(pool_alloc(r, (void**)&d_codes, (size_t)n_q * B * Tf * sizeof(int64_t)));
-    FCB_CK(cudaMemcpyAsync(d_wav, wav_host, (size_t)B * L * sizeof(float), cudaMemcpyHostToDevice, st));
+    FCB_CK(cudaMemcpyAsync(d_wav, wav_host, n_wav * sizeof(float), cudaMemcpyHostToDevice, st));
     int rc = fcb_roundtrip(h, d_wav, B, L, n_q, use_scale, d_codes, nullptr, nullptr, nullptr, d_recon, stream);
     if (rc == FCB_OK) {
         FCB_CK(cudaMemcpyAsync(codes_host, d_codes, (size_t)n_q * B * Tf * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-        FCB_CK(cudaMemcpyAsync(recon_host, d_recon, (size_t)B * L * sizeof(float), cudaMemcpyDeviceToHost, st));
+        FCB_CK(cudaMemcpyAsync(recon_host, d_recon, n_wav * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
     FCB_TRY(pool_free(r, d_wav));
     FCB_TRY(pool_free(r, d_recon));
@@ -1811,6 +1826,7 @@ int fcb_debug_conv1d(fcb_handle* h, const char* layer, const float* x, int32_t B
     Run r{h, B, (cudaStream_t)stream};
     Act in;
     in.p = const_cast<float*>(x); in.T = T; in.C = L->cin; in.clip_stride = (long long)T * L->cin;
+    if (L == &h->enc_conv0 && L->cin > 1) in.ch_stride = T;      // the stereo first conv reads the planar waveform layout
     Act o;
     FCB_TRY(run_conv(r, in, nullptr, elu != 0, nullptr, *L, stats != nullptr, &o));
     const long long rows = o.clip_stride / o.C;

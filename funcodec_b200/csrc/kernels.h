@@ -16,11 +16,12 @@ cudaError_t launch_conv(const ConvParams& p, int B, cudaStream_t st, int* nparts
 cudaError_t launch_stats_finalize(const double* partials, int nparts, double count, float eps, int mode,
                                   float* out, int B, cudaStream_t st, const float* gamma = nullptr,
                                   const float* beta = nullptr, int C = 0, float* coef = nullptr);
-bool conv_cout1_supported(const ConvParams& p);
-int conv_cout1_num_parts(int T_out);
+bool conv_cout1_supported(const ConvParams& p);          // C_out 1 or 2 (mono / stereo decoder output conv)
+int conv_cout1_num_parts(int T_out, int C_out);
 cudaError_t launch_conv_cout1(const ConvParams& p, int B, cudaStream_t st, int* nparts);
 int sumsq_num_parts(int L);
-cudaError_t launch_sumsq_partials(const float* x, int B, int L, double* partials, int* nparts, cudaStream_t st);
+// C = 2: planar stereo clips [B][2][L], squares of the mono mix (x0 + x1) / 2
+cudaError_t launch_sumsq_partials(const float* x, int B, int L, double* partials, int* nparts, cudaStream_t st, int C = 1);
 
 // conv_tc.cu
 bool conv_tc_supported(int C_in, int C_out_eff, int K, int S, int D);
@@ -88,9 +89,11 @@ cudaError_t launch_embed_sum(const long long* codes, int q_major, const float* e
                              float* out, int* err_flag, cudaStream_t st);
 
 // misc.cu
+// raw [B][T_raw][C] channels-last -> out [B][C][out_len] planar, C in {1, 2}
 cudaError_t launch_final_output(const float* raw, const float* stats, const float* gamma, const float* beta,
-                                const float* scale, int B, int T_raw, int out_len, float* out, cudaStream_t st);
+                                const float* scale, int B, int T_raw, int out_len, float* out, cudaStream_t st, int C = 1);
 cudaError_t launch_fill(float* p, float v, long long n, cudaStream_t st);
+// planar multi-channel clips [B][C][L] are B*C rows here (segments [(s*B + b)][C][seg_len]); launch_overlap_add likewise
 cudaError_t launch_gather_segments(const float* wav, int B, int L, int seg_len, int stride, int s0, int n_seg, float* out,
                                    cudaStream_t st);
 constexpr int OLA_MAX_TAILS = 16;

@@ -23,22 +23,27 @@ cudaError_t ensure_dynamic_smem(const void* kernel, int bytes) {
     return e;
 }
 
-// Final GroupNorm(1,1) of the decoder's last conv (seanet_decoder.py:160-164 -> conv.py:162), optional
-// `out * scale` (codec_basic.py:405-407) and the `[:, :, :L]` trim (codec_basic.py:711) in one pass.
+// Final GroupNorm(1, C) of the decoder's last conv (seanet_decoder.py:160-164 -> conv.py:162), optional
+// `out * scale` (codec_basic.py:405-407) and the `[:, :, :L]` trim (codec_basic.py:711) in one pass.  The raw conv output is
+// channels-last [B][T_raw][C]; the waveform is written channel-planar [B][C][out_len] (C = 2: stereo, one scale per clip).
+template <int C>
 __global__ void final_output_kernel(const float* __restrict__ raw, const float* __restrict__ stats,
                                     const float* __restrict__ gamma, const float* __restrict__ beta,
                                     const float* __restrict__ scale, int T_raw, int out_len, float* __restrict__ out) {
     const int b = blockIdx.y;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= out_len) return;
-    float v = raw[(long long)b * T_raw + t];
-    if (stats) {       // deferred GroupNorm(1, 1) of the last conv (norm: time_group_norm); weight_norm / none output is plain
-        const float mean = stats[2 * b], rstd = stats[2 * b + 1];
-        const float a = rstd * gamma[0];
-        v = fmaf(v, a, beta[0] - a * mean);
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+        float v = raw[((long long)b * T_raw + t) * C + c];
+        if (stats) {   // deferred GroupNorm(1, C) of the last conv (norm: time_group_norm); weight_norm / none output is plain
+            const float mean = stats[2 * b], rstd = stats[2 * b + 1];
+            const float a = rstd * gamma[c];
+            v = fmaf(v, a, beta[c] - a * mean);
+        }
+        if (scale) v = v * scale[b];
+        out[((long long)b * C + c) * out_len + t] = v;
     }
-    if (scale) v = v * scale[b];
-    out[(long long)b * out_len + t] = v;
 }
 
 __global__ void fill_kernel(float* p, float v, long long n) {
@@ -47,12 +52,17 @@ __global__ void fill_kernel(float* p, float v, long long n) {
 }
 
 cudaError_t launch_final_output(const float* raw, const float* stats, const float* gamma, const float* beta,
-                                const float* scale, int B, int T_raw, int out_len, float* out, cudaStream_t st) {
-    final_output_kernel<<<dim3((out_len + 255) / 256, B), 256, 0, st>>>(raw, stats, gamma, beta, scale, T_raw, out_len, out);
+                                const float* scale, int B, int T_raw, int out_len, float* out, cudaStream_t st, int C) {
+    if (C == 2)
+        final_output_kernel<2><<<dim3((out_len + 255) / 256, B), 256, 0, st>>>(raw, stats, gamma, beta, scale, T_raw, out_len, out);
+    else
+        final_output_kernel<1><<<dim3((out_len + 255) / 256, B), 256, 0, st>>>(raw, stats, gamma, beta, scale, T_raw, out_len, out);
     return cudaGetLastError();
 }
 
 // ---- segment_dur != None (Encodec._encode / _decode, codec_basic.py:334-359,382-396)
+// A planar multi-channel batch [B][C][L] is passed as B*C single-channel rows: the gathered segments are then
+// [(s*B + b)][C][seg_len], and the overlap-add applies the same triangular weights to every channel (codec_basic.py:77-116).
 // Segments as a batch: out[(s*B + b)][j] = wav[b][(s0 + s)*stride + j], j < seg_len (every gathered segment is full length).
 __global__ void gather_segments_kernel(const float* __restrict__ wav, int B, int L, int seg_len, int stride, int s0,
                                        float* __restrict__ out) {

@@ -63,13 +63,15 @@ class B200Encodec:
         c.conv_group_ratio, c.tr_conv_group_ratio = cfg.conv_group_ratio, cfg.tr_conv_group_ratio
         c.n_residual_layers, c.dilation_base = cfg.n_residual_layers, cfg.dilation_base
         c.norm, c.causal = NORM_CODES[cfg.norm], int(cfg.causal)
+        c.channels = cfg.channels
         for i, r in enumerate(cfg.ratios_f):
             c.ratios_f[i] = r
         self._h = ctypes.c_void_p()
         with torch.cuda.device(self.device):
             rc = self._lib.fcb_create(ctypes.byref(c), ctypes.byref(self._h))
             if rc != 0:
-                raise _capi.FcbError(f"fcb_create failed (rc={rc})")
+                why = " (stereo is built for the time-domain Encodec only)" if cfg.channels == 2 and cfg.arch != 0 else ""
+                raise _capi.FcbError(f"fcb_create failed (rc={rc}){why}")
             for key, val in (options or {}).items():
                 _capi.check(self._lib, self._h, self._lib.fcb_set_option(self._h, key.encode(), int(val)),
                             f"fcb_set_option({key})")
@@ -118,9 +120,11 @@ class B200Encodec:
 
     def debug_conv(self, layer: str, x_btc: torch.Tensor, elu: bool = False, want_stats: bool = True):
         """fcb_debug_conv1d test hook: one packed layer on a plain channels-last input -> (raw y [B,t_out,c_out],
-        stats [B,2] | None, row_off)."""
+        stats [B,2] | None, row_off).  The stereo first conv takes the waveform's planar layout, so x is transposed for it."""
+        B, T, Cx = x_btc.shape
+        if layer == "encoder.model.0" and Cx > 1:
+            x_btc = x_btc.transpose(1, 2)
         x = x_btc.to(self.device, torch.float32).contiguous()
-        B, T, _ = x.shape
         cap = B * (T + 2) * 8192
         y = torch.empty(cap, dtype=torch.float32, device=self.device)
         stats = torch.empty((B, 2), dtype=torch.float32, device=self.device) if want_stats else None
@@ -150,14 +154,14 @@ class B200Encodec:
     def _inference_segmented(self, x: torch.Tensor, need_recon: bool, n_q: int, use_scale: bool):
         """Encodec.inference with segment_dur != None (codec_basic.py:334-359,382-396,695-718): one list entry per segment,
         recon_speech = linear overlap-add of the decoded segments trimmed to L.  sub_quants are not produced here."""
-        B, L = x.shape
+        B, L = x.shape[0], x.shape[-1]
         plan = self.plan_segments(L)
         D, dev = self.cfg.dimension, self.device
         nf, T0 = plan.n_full, plan.frames_full
         codes = torch.empty(n_q * B * plan.total_frames, dtype=torch.int64, device=dev)
         quant = torch.empty(B * plan.total_frames * D, dtype=torch.float32, device=dev)
         scale = torch.empty((plan.n_seg, B, 1), dtype=torch.float32, device=dev)
-        recon = torch.empty((B, 1, L), dtype=torch.float32, device=dev) if need_recon else None
+        recon = torch.empty((B, self.cfg.channels, L), dtype=torch.float32, device=dev) if need_recon else None
         with torch.cuda.device(dev):
             self._ck(self._lib.fcb_roundtrip_segmented(self._h, _ptr(x), B, L, self.segment_length, self.segment_stride, n_q,
                                                        int(use_scale), _ptr(codes), _ptr(quant), _ptr(scale), _ptr(recon),
@@ -205,6 +209,11 @@ class B200Encodec:
         return y[:B * F_raw * T_raw * Co].view(B, F_raw, T_raw, Co), stats, (f_off, t_off, Fl, Tl)
 
     def _prep_speech(self, speech: torch.Tensor) -> torch.Tensor:
+        """-> [B, L] for a mono model, channel-planar [B, 2, L] for a stereo one (the reference's [B, C, L] layout)."""
+        if self.cfg.channels == 2:
+            if speech.dim() != 3 or speech.shape[1] != 2:
+                raise ValueError(f"this model is stereo (input_size: 2): speech must be [B, 2, L], got {tuple(speech.shape)}")
+            return speech.to(self.device, torch.float32).contiguous()
         if speech.dim() == 3:
             if speech.shape[1] != 1:
                 raise ValueError("only mono input is supported (input_size: 1)")
@@ -220,7 +229,8 @@ class B200Encodec:
         """Encodec.inference (codec_basic.py:670-718).  `need_sub_quants=False` skips the [n_q,B,D,T'] tensor
         (the reference always builds it; codec_inference.py only reads it under --need_sub_quants)."""
         x = self._prep_speech(speech)
-        B, L = x.shape
+        B, L = x.shape[0], x.shape[-1]
+        C = self.cfg.channels
         Tf = self.num_frames(L)
         # the reference slices self.layers[:n_q] (ddp_core_vq.py:386): a bandwidth above the maximum uses every stage
         n_q = min(self.cfg.num_quantizers_for_bandwidth(bit_width), self.cfg.num_quantizers)
@@ -239,14 +249,14 @@ class B200Encodec:
         Lr = min(L, self.cfg.decoded_length(Tf))
         with torch.cuda.device(dev):
             if need_recon and not need_encoder_out and Lr == L:
-                recon = torch.empty((B, 1, L), dtype=torch.float32, device=dev)
+                recon = torch.empty((B, C, L), dtype=torch.float32, device=dev)
                 self._ck(self._lib.fcb_roundtrip(self._h, _ptr(x), B, L, n_q, int(use_scale), _ptr(codes), _ptr(quant),
                                                  _ptr(scale), _ptr(sub), _ptr(recon), self._stream()), "fcb_roundtrip")
             else:
                 self._ck(self._lib.fcb_encode(self._h, _ptr(x), B, L, n_q, _ptr(codes), _ptr(quant), _ptr(scale),
                                               _ptr(sub), _ptr(enc), self._stream()), "fcb_encode")
                 if need_recon:
-                    recon = torch.empty((B, 1, Lr), dtype=torch.float32, device=dev)
+                    recon = torch.empty((B, C, Lr), dtype=torch.float32, device=dev)
                     sc = scale if (use_scale and self.audio_normalize) else None
                     self._ck(self._lib.fcb_decode_emb(self._h, _ptr(quant), B, Tf, _ptr(sc), _ptr(recon), Lr,
                                                       self._stream()), "fcb_decode_emb")
@@ -274,7 +284,7 @@ class B200Encodec:
         B, Tf, n_q = tok.shape
         D, Lo = self.cfg.dimension, self.cfg.decoded_length(Tf)
         emb = torch.empty((B, Tf, D), dtype=torch.float32, device=self.device)
-        recon = torch.empty((B, 1, Lo), dtype=torch.float32, device=self.device)
+        recon = torch.empty((B, self.cfg.channels, Lo), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
             self._ck(self._lib.fcb_decode_codes(self._h, _ptr(tok), B, Tf, n_q, _ptr(emb), _ptr(recon), Lo,
                                                 self._stream()), "fcb_decode_codes")
@@ -295,7 +305,7 @@ class B200Encodec:
         Lo = self.cfg.decoded_length(Tf)
         recon = None
         if need_recon:
-            recon = torch.empty((B, 1, Lo), dtype=torch.float32, device=self.device)
+            recon = torch.empty((B, self.cfg.channels, Lo), dtype=torch.float32, device=self.device)
             with torch.cuda.device(self.device):
                 self._ck(self._lib.fcb_decode_emb(self._h, _ptr(emb), B, Tf, None, _ptr(recon), Lo,
                                                   self._stream()), "fcb_decode_emb")
@@ -305,8 +315,10 @@ class B200Encodec:
     @torch.no_grad()
     def roundtrip_host(self, wav_pinned: torch.Tensor, codes_pinned: torch.Tensor, recon_pinned: torch.Tensor,
                        bit_width: int = None, use_scale: bool = True):
-        """fcb_roundtrip_host: HOST (pinned) buffers in and out, copies inside the call, synchronous."""
-        B, L = wav_pinned.shape
+        """fcb_roundtrip_host: HOST (pinned) buffers in and out, copies inside the call, synchronous.  wav / recon are
+        [B, L] (mono) or [B, 2, L] (stereo)."""
+        B, L = wav_pinned.shape[0], wav_pinned.shape[-1]
+        assert wav_pinned.numel() == B * self.cfg.channels * L and recon_pinned.numel() == wav_pinned.numel()
         n_q = min(self.cfg.num_quantizers_for_bandwidth(bit_width), self.cfg.num_quantizers)
         assert codes_pinned.shape == (n_q, B, self.num_frames(L)) and codes_pinned.dtype == torch.int64
         assert recon_pinned.shape[0] == B and recon_pinned.shape[-1] == L

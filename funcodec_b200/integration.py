@@ -84,6 +84,12 @@ def config_from_reference_model(model) -> CodecConfig:
             raise UnsupportedReferenceModel(f"residual-block dilations {dils} are not dilation_base ** j")
     if n_res > 1 and freq:
         raise UnsupportedReferenceModel("n_residual_layers > 1 is only supported for the time-domain stacks")
+    # audio channels: SEANetEncoder.channels = input_size, SEANetDecoder.channels (seanet_encoder.py:98, seanet_decoder.py:101)
+    channels = int(getattr(enc, "channels", 1) or 1) if not freq else 1
+    if not freq and channels != int(getattr(dec, "channels", 1) or 1):
+        raise UnsupportedReferenceModel(f"encoder channels {channels} != decoder channels {getattr(dec, 'channels', 1)}")
+    if channels not in (1, 2):
+        raise UnsupportedReferenceModel(f"{channels} audio channels: mono or stereo only (codec_basic.py:342-344)")
     dconf = getattr(model, "domain_conf", None) or {}
     cfg = CodecConfig(name="from_reference", ratios=ratios, arch=1 if freq else 0, ratios_f=ratios_f,
                       n_fft=int(dconf.get("n_fft", 512)), stft_hop=int(dconf.get("hop_length", 160)),
@@ -93,7 +99,7 @@ def config_from_reference_model(model) -> CodecConfig:
                       residual_kernel_size=int(rb_k), lstm_layers=n_lstm, codebook_size=int(embed.shape[1]),
                       num_quantizers=int(embed.shape[0]), sample_rate=int(q.sampling_rate),
                       audio_normalize=bool(model.audio_normalize), n_residual_layers=n_res, dilation_base=dil_base,
-                      norm=norm, causal=causal)
+                      norm=norm, causal=causal, channels=channels)
     if cfg.hop_length != int(q.encoder_hop_length):
         raise UnsupportedReferenceModel("quantizer.encoder_hop_length does not match prod(ratios)")
     if freq:

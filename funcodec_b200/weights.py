@@ -23,7 +23,7 @@ def conv_specs(cfg: CodecConfig) -> List[Dict]:
                 dict(name=prefix + ".block.3.conv", kind="conv", cin=dim // 2, cout=dim, k=1, s=1),
                 dict(name=prefix + ".shortcut.conv", kind="conv", cin=dim, cout=dim, k=1, s=1)]
 
-    specs.append(dict(name="encoder.model.0.conv", kind="conv", cin=1, cout=nf, k=cfg.kernel_size, s=1))
+    specs.append(dict(name="encoder.model.0.conv", kind="conv", cin=cfg.channels, cout=nf, k=cfg.kernel_size, s=1))
     n, mult = 1, 1
     nres = cfg.n_residual_layers
     for r in reversed(cfg.ratios):
@@ -48,7 +48,7 @@ def conv_specs(cfg: CodecConfig) -> List[Dict]:
             specs += rb(f"decoder.model.{n + 2 + j}", mult * nf // 2)
         mult //= 2
         n += nres + 2
-    specs.append(dict(name=f"decoder.model.{n + 1}.conv", kind="conv", cin=nf, cout=1, k=cfg.last_kernel_size, s=1))
+    specs.append(dict(name=f"decoder.model.{n + 1}.conv", kind="conv", cin=nf, cout=cfg.channels, k=cfg.last_kernel_size, s=1))
     return specs
 
 

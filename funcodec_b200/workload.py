@@ -9,6 +9,7 @@ is what `--stat_flops` logs in place of the reference's thop profile (codec_infe
   * layer-boundary bytes: 4 * (|module input| + |module output|) per conv / transposed-conv MODULE as the hooks see them: the
     conv input is the padded tensor (SConv pads before calling the conv), the transposed-conv output is the untrimmed one
   * LSTM MACs: 2 stacks x layers x T' x 8 H^2 (W_ih and W_hh, 4 gates);  RVQ FLOPs: 2 * T' * n_q * K * D
+  * stereo (cfg.channels = 2): the first conv reads and the last conv writes 2 channels per sample; L counts samples per channel
 """
 from typing import Dict
 
@@ -39,7 +40,7 @@ def _time_stacks(cfg: CodecConfig, L: int, layers=None):
         for l in range(cfg.lstm_layers):
             note(f"{side}.lstm.ih_l{l}", H, 4 * H, 1, 1, T, T * H * 4 * H, 4 * (T * H + T * 4 * H))
 
-    T = conv(1, nf, cfg.kernel_size, 1, L, name="enc.conv0")
+    T = conv(cfg.channels, nf, cfg.kernel_size, 1, L, name="enc.conv0")
     mult = 1
     for i, r in enumerate(reversed(cfg.ratios)):
         for j in range(nres):
@@ -66,7 +67,7 @@ def _time_stacks(cfg: CodecConfig, L: int, layers=None):
             conv(cout // 2, cout, 1, 1, T, name=f"dec.{i}.rb{j}.1x1")
             conv(cout, cout, 1, 1, T, name=f"dec.{i}.rb{j}.shortcut")
         mult //= 2
-    conv(nf, 1, cfg.last_kernel_size, 1, T, name="dec.final")
+    conv(nf, cfg.channels, cfg.last_kernel_size, 1, T, name="dec.final")
     return macs, byts, params, frames, H
 
 

@@ -15,7 +15,8 @@
  *   - every call is asynchronous on `stream` (no host synchronisation) unless stated otherwise.
  *   - return value: 0 = OK, negative = error (FCB_E_*); fcb_last_error() gives the text.  No C++
  *     exception crosses the ABI.  One handle per caller thread/stream; handles are not internally locked.
- *   - tensors use the reference's user-facing layouts: wav [B, L] fp32; codes int64
+ *   - tensors use the reference's user-facing layouts: wav [B, L] fp32 ([B, 2, L] channel-planar for a stereo handle,
+ *     fcb_config.channels = 2: every wav / wav_out / recon buffer below then holds 2 * L samples per clip); codes int64
  *     [n_q, B, T'] (encode side) and [B, T', n_q] (decode side, codec_basic.py:789); embeddings
  *     [B, T', D] fp32; sub_quants [n_q, B, D, T'] fp32.
  */
@@ -82,6 +83,13 @@ typedef struct fcb_config {
      * causal with time_group_norm is refused like the reference does (conv.py:46-47); arch 1 takes neither. */
     int32_t norm;
     int32_t causal;
+    /* Audio channels of the time-domain stacks (arch 0): 0 or 1 mono, 2 stereo (Encodec input_size / SEANetDecoder channels;
+     * _encode asserts 0 < channels <= 2, codec_basic.py:342-344).  A stereo handle takes and returns every waveform buffer in
+     * the reference's channel-planar layout [B, 2, L]; the RMS scale is one value per clip, taken from the mono mix
+     * x.mean(dim=1) (:366-369).  The first encoder conv then has 2 input channels ("encoder.model.0.conv.conv.weight"
+     * [n_filters, 2, k]) and the last decoder conv 2 output channels (weight [2, n_filters, k], bias and GroupNorm affine [2]).
+     * arch 1 (FreqCodec, which STFTs x.squeeze(1)) is mono only: fcb_create refuses channels 2 there. */
+    int32_t channels;
 } fcb_config;
 
 typedef struct fcb_handle fcb_handle;
@@ -115,7 +123,7 @@ FCB_API int fcb_num_quantizers_for_bandwidth(const fcb_handle* h, double bandwid
 
 /* Encodec.inference_encoding (codec_basic.py:720-764) / the encode half of Encodec.inference:
  * RMS-normalise (:366-371) -> SEANetEncoder -> RVQ (ddp_core_vq.py:367-418).
- *   wav          dev [B, L] fp32
+ *   wav          dev [B, L] fp32 ([B, 2, L] stereo)
  *   codes        dev [n_q, B, T'] int64                               (required)
  *   quant        dev [B, T', D] fp32 quantized embeddings            (nullable)
  *   scale        dev [B] fp32 per-clip RMS scale (1.0 when !audio_normalize)   (nullable)
@@ -127,7 +135,7 @@ FCB_API int fcb_encode(fcb_handle* h, const float* wav, int32_t B, int32_t L, in
 
 /* Encodec.inference_decoding_emb (codec_basic.py:804-836) and the decode half of Encodec.inference
  * (:709-711): SEANetDecoder -> optional * scale -> keep the first out_len samples.
- *   emb dev [B, T', D]; scale dev [B] or NULL; wav_out dev [B, out_len], out_len <= T' * hop. */
+ *   emb dev [B, T', D]; scale dev [B] or NULL; wav_out dev [B, out_len] ([B, 2, out_len] stereo), out_len <= T' * hop. */
 FCB_API int fcb_decode_emb(fcb_handle* h, const float* emb, int32_t B, int32_t n_frames, const float* scale,
                    float* wav_out, int32_t out_len, void* stream);
 
@@ -144,7 +152,7 @@ FCB_API int fcb_decode_codes(fcb_handle* h, const int64_t* codes, int32_t B, int
 FCB_API int fcb_check_errors(fcb_handle* h, void* stream);
 
 /* Encodec.inference (codec_basic.py:670-718) with need_recon=True in one call: fcb_encode followed by
- * decode of the quantized embeddings, recon dev [B, L].  use_scale as in the reference. */
+ * decode of the quantized embeddings, recon dev [B, L] ([B, 2, L] stereo).  use_scale as in the reference. */
 FCB_API int fcb_roundtrip(fcb_handle* h, const float* wav, int32_t B, int32_t L, int32_t n_q, int32_t use_scale,
                   int64_t* codes, float* quant, float* scale, float* sub_quants, float* recon,
                   void* stream);
@@ -178,7 +186,8 @@ FCB_API int fcb_plan_segments_for_hop(int32_t hop, int32_t L, int32_t seg_len, i
  *   codes  int64: [n_q][n_full*B][frames_full] followed, per tail i, by [n_q][B][tail_frames[i]]
  *   quant  fp32 or NULL: [n_full*B][frames_full][D] followed by [B][tail_frames[i]][D] per tail
  *   scale  fp32 or NULL: [n_seg][B]
- *   recon  fp32 or NULL: [B][L] (NULL = encode only, Encodec.inference_encoding) */
+ *   recon  fp32 or NULL: [B][L], [B][2][L] stereo (NULL = encode only, Encodec.inference_encoding)
+ * wav is [B][L] ([B][2][L] stereo); every segment of a stereo clip gets one scale from its mono mix. */
 FCB_API int fcb_roundtrip_segmented(fcb_handle* h, const float* wav, int32_t B, int32_t L, int32_t seg_len, int32_t stride,
                                     int32_t n_q, int32_t use_scale, int64_t* codes, float* quant, float* scale,
                                     float* recon, void* stream);
@@ -210,7 +219,8 @@ FCB_API int fcb_set_option(fcb_handle* h, const char* key, int32_t value);
 
 /* TEST HOOK (tests/test_gpu_layers.py): run ONE packed conv layer, addressed by its reference module prefix
  * ("encoder.model.3", "decoder.model.3", "encoder.model.1.block.1", "encoder.model.16.lstm.ih0", ...), on a plain
- * channels-last input x dev [B][T][C_in] (optional ELU on load).  y dev receives the RAW output (bias added,
+ * channels-last input x dev [B][T][C_in] (optional ELU on load; "encoder.model.0" of a stereo handle reads x channel-planar
+ * [B][2][T] like fcb_encode's waveform).  y dev receives the RAW output (bias added,
  * GroupNorm not applied) as [B][t_out][c_out] where for a transposed conv t_out is the UNtrimmed length and
  * row_off the first kept row (conv.py:299-303); stats dev [B][2] = (mean, rstd) of the layer's GroupNorm or NULL. */
 FCB_API int fcb_debug_conv1d(fcb_handle* h, const char* layer, const float* x, int32_t B, int32_t T, int32_t elu,

@@ -38,7 +38,8 @@ def build_reference_encodec(cfg):
     discriminator; cfg is a funcodec_b200.config.CodecConfig."""
     import torch
     Encodec, SEANetEncoder, SEANetDecoder, CostumeQuantizer = import_reference()
-    enc = SEANetEncoder(input_size=1, dimension=cfg.dimension, n_filters=cfg.n_filters,
+    channels = getattr(cfg, "channels", 1)       # input_size / decoder_conf.channels (2: stereo)
+    enc = SEANetEncoder(input_size=channels, dimension=cfg.dimension, n_filters=cfg.n_filters,
                         ratios=list(cfg.ratios), norm=getattr(cfg, "norm", "time_group_norm"), causal=bool(getattr(cfg, "causal", False)),
                         kernel_size=cfg.kernel_size, last_kernel_size=cfg.last_kernel_size,
                         residual_kernel_size=cfg.residual_kernel_size,
@@ -49,13 +50,13 @@ def build_reference_encodec(cfg):
                              sampling_rate=cfg.sample_rate, quantize_dropout=True,
                              rand_num_quant=[2, 4, 8, 16, 32], use_ddp=True,
                              encoder_hop_length=cfg.hop_length)
-    dec = SEANetDecoder(input_size=cfg.dimension, channels=1, n_filters=cfg.n_filters,
+    dec = SEANetDecoder(input_size=cfg.dimension, channels=channels, n_filters=cfg.n_filters,
                         ratios=list(cfg.ratios), norm=getattr(cfg, "norm", "time_group_norm"), causal=bool(getattr(cfg, "causal", False)),
                         kernel_size=cfg.kernel_size, last_kernel_size=cfg.last_kernel_size,
                         residual_kernel_size=cfg.residual_kernel_size,
                         seq_layer_num=cfg.lstm_layers, seq_model="lstm" if cfg.lstm_layers > 0 else "none",
                         n_residual_layers=cfg.n_residual_layers, dilation_base=cfg.dilation_base)
-    model = Encodec(input_size=1, odim=cfg.dimension, encoder=enc, quantizer=quant, decoder=dec,
+    model = Encodec(input_size=channels, odim=cfg.dimension, encoder=enc, quantizer=quant, decoder=dec,
                     discriminator=None, target_sample_hz=cfg.sample_rate,
                     multi_spectral_window_powers_of_two=[], audio_normalize=cfg.audio_normalize,
                     segment_dur=None, overlap_ratio=None)
